@@ -21,12 +21,18 @@ slot pipeline the way consecutive seconds of a video do, and the timed region is
                 duration with the pipeline full
   workloads     the same measurements for BASELINE.json configs[2] / [3]: the 4K (3840x2160, 16-bit depth) clip,
                 frame-sharded over the N GPUs like the headline; and for one corner of configs[4]: 8K VR frames with
-                maximum disparity and aggressive hole filling (3 steps of 16 frames at most)
+                maximum disparity and aggressive hole filling (16 frames per step)
   driver        frames/s of the drop-in frame loop on a synthetic workflow directory of real PNG files (rank 0, N = 1)
   cpu_baseline  the reference's CPU path timed on this box's host cores, bounded sample (rank 0, N = 1 only)
 --impl reference times the reference's own CPU implementation alone: the UNMODIFIED helper/stereo_core.py staged
 under oracle/_ref by oracle/make_ref.py (cpu_baseline.kind "reference"; every timed step one full 1080p frame), or,
 where that copy is absent, the oracle's C port of it (kind "port").
+
+--dump-outputs DIR writes, after the timed steps, what the device-resident leg of every workload returned in its last
+timed step (rank 0): `<workload>_sbs_sample.npy` (float32 [frames, DUMP_SAMPLES], the SBS uint8 values at fixed seeded
+positions of each distinct frame of that step), `<workload>_frames.npy` (the rows' distinct synthetic frames, i.e. their
+make_pair seeds) and `<workload>_sample_index.npy` (the positions, flat indices into the [H, 2W, 3] frame).  Inputs and
+positions depend on the arguments only, so two builds run with the same arguments can be compared value for value.
 """
 from __future__ import annotations
 
@@ -121,8 +127,28 @@ def make_frames(n, h, w, dtype, seed0=0):
     return [make_pair(h, w, seed0 + i, dtype) for i in range(n)]
 
 
+# 1 % of a 1080p SBS frame; at most 48 + 16 + 6 distinct frames of the three workloads: 37 MB of float32 samples plus
+# 3 MB of positions, inside the 64 MB a dump may take
+DUMP_SAMPLES = 1 << 17
+DUMP_SEED = 20240
+
+
+def dump_outputs(dump_dir, key, outs):
+    """Write a fixed, seeded sample of the SBS frames `outs` ({frame index: uint8 [H, 2W, 3] CUDA tensor})."""
+    import torch
+    frames = sorted(outs)
+    n = outs[frames[0]].numel()
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_SAMPLES), replace=False))
+    d_idx = torch.from_numpy(idx).to(outs[frames[0]].device)
+    sample = torch.stack([outs[f].reshape(-1)[d_idx] for f in frames]).float().cpu().numpy()
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, f'{key}_sbs_sample.npy'), sample)
+    np.save(os.path.join(dump_dir, f'{key}_frames.npy'), np.array(frames, np.float64))
+    np.save(os.path.join(dump_dir, f'{key}_sample_index.npy'), idx.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
-def run_workload(key, batch, slots, group, steps, warmup, rank, world, local_rank, dist, profile):
+def run_workload(key, batch, slots, group, steps, warmup, rank, world, local_rank, dist, profile, dump_dir=None):
     """Device-resident leg, end-to-end leg and (rank 0) the per-kernel profile of one workload."""
     import torch
     from vsc_b200 import StereoGenerator, StereoParams, _lib
@@ -150,6 +176,8 @@ def run_workload(key, batch, slots, group, steps, warmup, rank, world, local_ran
         def __init__(self):
             self.free, self.busy, self.last = list(range(slots)), [], None
 
+    written = {}        # (slot, k) -> (step, frame) last submitted into d_out[slot][k]
+
     def device_step(step, pipe):
         """one batch, inputs resident in HBM; a finished slot is reused at once (no head-of-line blocking);
         every submission carries `group` frames that share the slot's stream and one hole-filling launch"""
@@ -164,6 +192,7 @@ def run_workload(key, batch, slots, group, steps, warmup, rank, world, local_ran
             for k in range(min(group, batch - i0)):
                 f = (step * batch + i0 + k) % n_distinct
                 tri.append((d_rgb[f].data_ptr(), d_dep[f].data_ptr(), d_out[s][k].data_ptr()))
+                written[(s, k)] = (step, f)
             gen.submit_device_group(s, tri, DT, H, W, params)
             pipe.busy.append(s)
 
@@ -225,8 +254,13 @@ def run_workload(key, batch, slots, group, steps, warmup, rank, world, local_ran
         device_step(k, wp)
     device_drain(wp)
     launches_per_frame = gen.last_frame_launches(0) / group
+    written.clear()
     with ClockSampler(local_rank) as clk:
         ms_dev, wall_dev = timed(device_step, device_drain, steps)
+    if dump_dir is not None and rank == 0:
+        # d_out is reused within a step: the last step's frames whose buffers still hold them (with the default
+        # arguments, every distinct frame)
+        dump_outputs(dump_dir, key, {f: d_out[s][k] for (s, k), (st, f) in written.items() if st == steps - 1})
     wp = Pipe()
     for k in range(max(1, warmup // 2)):
         e2e_step(k, wp)
@@ -322,13 +356,15 @@ def run_ours(args, rank, world, local_rank):
     if world > 1:
         import torch.distributed as dist
         dist.init_process_group('nccl', device_id=torch.device('cuda', local_rank))
-    head = run_workload('1080p', args.batch, args.slots, args.group, args.steps, args.warmup, rank, world, local_rank, dist, True)
+    dump = args.dump_outputs
+    head = run_workload('1080p', args.batch, args.slots, args.group, args.steps, args.warmup, rank, world, local_rank, dist, True, dump)
     extra = None
     if not args.no_4k:
-        extra = run_workload('4k', args.batch_4k, args.slots_4k, args.group, args.steps, args.warmup, rank, world, local_rank, dist, True)
+        extra = run_workload('4k', args.batch_4k, args.slots_4k, args.group, args.steps, args.warmup, rank, world, local_rank, dist, True,
+                             dump)
     sweep = None
     if not args.no_8k:
-        sweep = run_workload('8k', 16, 4, 2, max(1, min(args.steps, 3)), 1, rank, world, local_rank, dist, True)
+        sweep = run_workload('8k', 16, 4, 2, args.steps, args.warmup, rank, world, local_rank, dist, True, dump)
     out = None
     if rank == 0:
         out = {'metric': head['metric'], 'value': head['value'], 'unit': 'frames/s', 'n_gpus': world, 'steps': args.steps,
@@ -536,7 +572,11 @@ def main():
     ap.add_argument('--cpu-frames', type=int, default=2, help='frames of the bounded CPU-baseline sample')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-driver', action='store_true', help='skip the file-based frame-loop measurement (driver)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help="write a seeded sample of each workload's last timed step's SBS "
+                                                          'frames to DIR/*.npy (rank 0)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

@@ -164,9 +164,11 @@ def test_sbs_sweep_cli(tmp_path):
 
 def test_bench_line_contract(tmp_path):
     """bench.py on a small configuration: one JSON line with the contract's keys (value, e2e with copy bytes, roofline
-    with measured kernel time, workloads, cpu_baseline of the staged reference or the port), and the launch count."""
+    with measured kernel time, workloads, cpu_baseline of the staged reference or the port), and the launch count; and the
+    --dump-outputs sample of the last timed step, whose values are the oracle's for the same frames."""
+    dump = tmp_path / 'dump'
     r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '1', '--warmup', '3', '--batch', '16', '--slots', '2',
-                        '--batch-4k', '4', '--slots-4k', '1', '--no-8k', '--no-driver', '--cpu-frames', '1'],
+                        '--batch-4k', '4', '--slots-4k', '1', '--no-8k', '--no-driver', '--cpu-frames', '1', '--dump-outputs', str(dump)],
                        capture_output=True, text=True, timeout=900, env=dict(os.environ, VSC_BENCH_NO_CLOCKS='1'))
     assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
     lines = [l for l in r.stdout.splitlines() if l.startswith('{')]
@@ -182,3 +184,14 @@ def test_bench_line_contract(tmp_path):
     w = d['workloads']['4k']
     assert w['value'] > 0 and w['e2e']['value'] > 0 and w['roofline']['algorithmic_bytes_per_launch'] % 91238400 == 0
     assert d['cpu_baseline']['kind'] in ('reference', 'port') and d['cpu_baseline']['value'] > 0
+    files = {p.name: np.load(p) for p in dump.iterdir()}
+    assert sorted(files) == sorted(f'{k}_{n}.npy' for k in ('1080p', '4k') for n in ('sbs_sample', 'frames', 'sample_index'))
+    assert all(a.dtype in (np.float32, np.float64) for a in files.values()) and sum(a.nbytes for a in files.values()) <= 64 << 20
+    for key, (fh, fw, dt, n_distinct) in {'1080p': (1080, 1920, np.uint8, 16), '4k': (2160, 3840, np.uint16, 4)}.items():
+        sample, frames, idx = (files[f'{key}_{n}.npy'] for n in ('sbs_sample', 'frames', 'sample_index'))
+        assert 0 < len(frames) <= n_distinct and set(frames) <= set(range(n_distinct))
+        assert np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < fh * 2 * fw * 3 and sample.shape == (len(frames), len(idx))
+        if key == '1080p':        # one frame of the timed path against the oracle
+            rgb, depth = make_pair(fh, fw, seed=int(frames[-1]), depth_dtype=dt)
+            ref = O.process_frame(rgb, depth, O.Params()).reshape(-1)[idx.astype(np.int64)]
+            assert np.array_equal(sample[-1], ref.astype(np.float32))
