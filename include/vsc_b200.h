@@ -123,6 +123,23 @@ int vsc_slot_elapsed_ms(vsc_ctx *ctx, int slot, float *ms);
 /* number of kernel launches issued for the last frame submitted on `slot` */
 int vsc_slot_launches(vsc_ctx *ctx, int slot);
 
+/* -------- output layouts (no reference counterpart) -------------------------------------------- */
+/* Every layout is a fixed function of the two final u8 eye images L, R [H,W,3] of the SBS layout:
+ *   SBS        [H,2W,3]  hstack(L, R)                        (the reference's output, the default)
+ *   HALF_SBS   [H,W,3]   hstack of both eyes at half width   (pixel pairs averaged, round half to even == cv2 INTER_AREA)
+ *   TB         [2H,W,3]  vstack(L, R), left eye on top
+ *   HALF_TB    [H,W,3]   vstack of both eyes at half height  (row pairs averaged, round half to even)
+ *   ANAGLYPH   [H,W,3]   Dubois least-squares red-cyan, float32 in a fixed order (DESIGN.md section 2)
+ * The half layouts take an even width (HALF_SBS) or height (HALF_TB) only. */
+enum { VSC_LAYOUT_SBS = 0, VSC_LAYOUT_HALF_SBS = 1, VSC_LAYOUT_TB = 2, VSC_LAYOUT_HALF_TB = 3, VSC_LAYOUT_ANAGLYPH = 4 };
+/* host only: output frame shape of a layout; VSC_E_INVALID for an unknown layout or an odd side a half layout halves */
+int vsc_layout_shape(int layout, int height, int width, int *out_h, int *out_w);
+/* layout of frames submitted to ctx from now on (vsc_process_frame, vsc_submit*, vsc_submit_device*);
+ * frames already in flight keep theirs.  Default VSC_LAYOUT_SBS.  out buffers must hold out_h*out_w*3 bytes.
+ * A submission whose frame size the layout cannot take fails with VSC_E_INVALID.  The layout adds no kernel launch:
+ * it is the store epilogue of the back-end kernel.  vsc_stage_backend always writes SBS. */
+int vsc_set_layout(vsc_ctx *ctx, int layout);
+
 /* -------- stage-level entry points for per-stage parity tests (host buffers, synchronous) --- */
 /* cv2.resize(src,(dst_w,H),INTER_LANCZOS4) (stereo_core.py:253-254); channels 1 or 3 for u8 */
 int vsc_stage_lanczos(vsc_ctx *ctx, const void *src, int dtype, int channels, int height, int width,

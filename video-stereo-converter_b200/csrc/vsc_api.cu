@@ -261,6 +261,7 @@ struct Slot {
     bool busy = false;
     const uint8_t* l_rgb = nullptr; const void* l_depth = nullptr; uint8_t* l_out = nullptr;
     int l_dtype = 0, l_H = 0, l_W = 0; vsc_params l_p; uint8_t* l_host_out = nullptr; size_t l_out_bytes = 0;
+    int l_layout = VSC_LAYOUT_SBS;       // output layout of the frame in this slot (fixed at submission)
     int launches = 0;
     float last_ms = 0.f;
     bool done = false;                   // leader only: the stream has run past the submission (set by a host callback)
@@ -276,6 +277,7 @@ struct vsc_ctx {
     int device = 0;
     int group_size = 1;                  // frames that share one stream and one hole-filling launch
     bool profiling = false;
+    int layout = VSC_LAYOUT_SBS;         // output layout of frames submitted from now on (vsc_set_layout)
     cudaStream_t tstream = nullptr;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     std::vector<cudaEvent_t> tslot;
@@ -343,6 +345,14 @@ static int upload_constants(vsc_ctx* ctx) {
     return VSC_OK;
 }
 
+template <int K>
+static int backend_attrs(int smem) {
+    const void* f[] = {(const void*)backend_kernel<K, VSC_LAYOUT_SBS>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_SBS>,
+                       (const void*)backend_kernel<K, VSC_LAYOUT_TB>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_TB>,
+                       (const void*)backend_kernel<K, VSC_LAYOUT_ANAGLYPH>};
+    for (const void* k : f) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    return VSC_OK;
+}
 static int set_smem_attrs() {
     const int big = 200 * 1024;
     CU(cudaFuncSetAttribute(lanczos_rgb_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
@@ -354,10 +364,8 @@ static int set_smem_attrs() {
     CU(cudaFuncSetAttribute(warp_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CU(cudaFuncSetAttribute(warp_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
     CU(cudaFuncSetAttribute(warp_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CU(cudaFuncSetAttribute(backend_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CU(cudaFuncSetAttribute(backend_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CU(cudaFuncSetAttribute(backend_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
-    CU(cudaFuncSetAttribute(backend_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, big));
+    int rc;
+    if ((rc = backend_attrs<0>(big)) || (rc = backend_attrs<2>(big)) || (rc = backend_attrs<3>(big)) || (rc = backend_attrs<4>(big))) return rc;
     CU(cudaFuncSetAttribute(telea_march_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MarchSh<16>)));
     CU(cudaFuncSetAttribute(telea_march_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MarchSh<32>)));
     return VSC_OK;
@@ -694,7 +702,19 @@ static int run_telea(vsc_ctx* ctx, Slot& s, int Hs, int Ws, const ViewSpec* vs, 
 #endif
     return VSC_OK;
 }
-static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4* v0, const uchar4* v1, uint8_t* d_out) {
+template <int K>
+static void launch_backend(int layout, dim3 grid, size_t smem, cudaStream_t st, const BackendArgs& a) {
+    switch (layout) {
+        case VSC_LAYOUT_HALF_SBS: backend_kernel<K, VSC_LAYOUT_HALF_SBS><<<grid, kThreads, smem, st>>>(a); break;
+        case VSC_LAYOUT_TB: backend_kernel<K, VSC_LAYOUT_TB><<<grid, kThreads, smem, st>>>(a); break;
+        case VSC_LAYOUT_HALF_TB: backend_kernel<K, VSC_LAYOUT_HALF_TB><<<grid, kThreads, smem, st>>>(a); break;
+        case VSC_LAYOUT_ANAGLYPH: grid.z = 1; backend_kernel<K, VSC_LAYOUT_ANAGLYPH><<<grid, kThreads, smem, st>>>(a); break;
+        default: backend_kernel<K, VSC_LAYOUT_SBS><<<grid, kThreads, smem, st>>>(a); break;
+    }
+}
+// d_out holds the frame in `layout` (vsc_layout_shape; the caller has checked that the layout takes H x W)
+static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4* v0, const uchar4* v1, uint8_t* d_out,
+                       int layout) {
     BackendArgs a;
     a.view[0] = v0; a.view[1] = v1; a.out = d_out;
     a.H = g.height; a.W = g.width; a.Hs = g.ss_h; a.Ws = g.ss_w;
@@ -713,11 +733,11 @@ static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4*
     if (smem > 200 * 1024) return fail(VSC_E_INVALID, "super_sampling too large for the back-end tile (%zu bytes of shared memory)", smem);
     dim3 grid((g.width + BE_OX - 1) / BE_OX, (g.height + BE_OY - 1) / BE_OY, 2);
     prof_begin(s, "backend_kernel");
-    switch (K) {
-        case 2: backend_kernel<2><<<grid, kThreads, smem, s.stream>>>(a); break;
-        case 3: backend_kernel<3><<<grid, kThreads, smem, s.stream>>>(a); break;
-        case 4: backend_kernel<4><<<grid, kThreads, smem, s.stream>>>(a); break;
-        default: backend_kernel<0><<<grid, kThreads, smem, s.stream>>>(a); break;
+    switch (K) {       // the anaglyph runs both eyes in one CTA (grid.z = 1)
+        case 2: launch_backend<2>(layout, grid, smem, s.stream, a); break;
+        case 3: launch_backend<3>(layout, grid, smem, s.stream, a); break;
+        case 4: launch_backend<4>(layout, grid, smem, s.stream, a); break;
+        default: launch_backend<0>(layout, grid, smem, s.stream, a); break;
     }
     KCHECK(s);
     return VSC_OK;
@@ -785,7 +805,7 @@ static int enqueue_group(vsc_ctx* ctx, Slot* fr, int n, int dtype, const vsc_geo
     int rc = run_telea(ctx, lead, g.ss_h, g.ss_w, vs, 2 * n);
     if (rc) return rc;
     for (int i = 0; i < n; i++)
-        if ((rc = run_backend(fr[i], g, p.sharpen, cur[2 * i], cur[2 * i + 1], fr[i].l_out))) return rc;
+        if ((rc = run_backend(fr[i], g, p.sharpen, cur[2 * i], cur[2 * i + 1], fr[i].l_out, fr[i].l_layout))) return rc;
     CU(cudaEventRecord(lead.ev1, lead.stream));
     for (int i = 0; i < n; i++)
         CU(cudaMemcpyAsync(fr[i].h_scalars, fr[i].scalars.p, sizeof(FrameScalars), cudaMemcpyDeviceToHost, lead.stream));
@@ -816,11 +836,15 @@ static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const
     vsc_geom g;
     int rc;
     if ((rc = vsc_geometry(H, W, p, &g))) return rc;
+    const int layout = ctx->layout;
+    int oh, ow;
+    if ((rc = vsc_layout_shape(layout, H, W, &oh, &ow))) return rc;
     CU(cudaSetDevice(ctx->device));
-    const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype), nout = (size_t)H * 2 * W * 3;
+    const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype), nout = (size_t)oh * ow * 3;
     for (int i = 0; i < n; i++) {
         Slot& s = fr[i];
         s.l_rgb = rgb[i]; s.l_depth = depth[i]; s.l_out = out[i]; s.l_host_out = nullptr; s.l_out_bytes = nout;
+        s.l_layout = layout;
         if (!device_io) {
             if (s.in_rgb.ensure(nrgb) || s.in_depth.ensure(ndepth) || s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
             CU(cudaMemcpyAsync(s.in_rgb.p, rgb[i], nrgb, cudaMemcpyHostToDevice, lead.stream));
@@ -955,6 +979,29 @@ extern "C" int vsc_slot_launches(vsc_ctx* ctx, int slot) {
     int total = 0;
     for (int i = 0; i < ctx->group_size; i++) total += fr[i].launches;
     return total;
+}
+
+extern "C" int vsc_layout_shape(int layout, int H, int W, int* out_h, int* out_w) {
+    if (!out_h || !out_w) return fail(VSC_E_INVALID, "null argument");
+    if (H < 1 || W < 1) return fail(VSC_E_INVALID, "bad frame size %dx%d", W, H);
+    switch (layout) {
+        case VSC_LAYOUT_SBS: *out_h = H; *out_w = 2 * W; return VSC_OK;
+        case VSC_LAYOUT_TB: *out_h = 2 * H; *out_w = W; return VSC_OK;
+        case VSC_LAYOUT_ANAGLYPH: *out_h = H; *out_w = W; return VSC_OK;
+        case VSC_LAYOUT_HALF_SBS:
+            if (W % 2) return fail(VSC_E_INVALID, "half-sbs halves the width: frame width %d is odd", W);
+            *out_h = H; *out_w = W; return VSC_OK;
+        case VSC_LAYOUT_HALF_TB:
+            if (H % 2) return fail(VSC_E_INVALID, "half-tb halves the height: frame height %d is odd", H);
+            *out_h = H; *out_w = W; return VSC_OK;
+        default: return fail(VSC_E_INVALID, "unknown output layout %d", layout);
+    }
+}
+extern "C" int vsc_set_layout(vsc_ctx* ctx, int layout) {
+    if (!ctx) return fail(VSC_E_INVALID, "null context");
+    if (layout < VSC_LAYOUT_SBS || layout > VSC_LAYOUT_ANAGLYPH) return fail(VSC_E_INVALID, "unknown output layout %d", layout);
+    ctx->layout = layout;
+    return VSC_OK;
 }
 
 extern "C" int vsc_process_frame(vsc_ctx* ctx, const uint8_t* rgb, const void* depth, int dtype, int H, int W,
@@ -1163,7 +1210,7 @@ extern "C" int vsc_stage_backend(vsc_ctx* ctx, const uint8_t* left, const uint8_
     if (!rc) rc = upload_view(s, right, nullptr, n, d1);
     if (rc) return rc;
     if (dout.alloc(nout)) return VSC_E_NOMEM;
-    if ((rc = run_backend(s, g, sharpen, (const uchar4*)d0.p, (const uchar4*)d1.p, (uint8_t*)dout.p))) return rc;
+    if ((rc = run_backend(s, g, sharpen, (const uchar4*)d0.p, (const uchar4*)d1.p, (uint8_t*)dout.p, VSC_LAYOUT_SBS))) return rc;
     CU(cudaMemcpyAsync(out_sbs, dout.p, nout, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
     return VSC_OK;

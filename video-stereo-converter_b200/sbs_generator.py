@@ -13,10 +13,14 @@ a carriage-return progress line on stdout that the orchestrator scrapes), but th
 and a frame-range sharder spreads one clip over the GPUs of the box (`--gpus N`, or launch under
 torchrun with one process per GPU).  Frames are independent, so there is no collective.
 There is no CPU path: `--cpu` is refused.
+
+`--layout` (or the top-level config.json key "sbs_layout") picks the output frame layout: the reference's full-width
+side-by-side (default), half side-by-side, top-bottom, half top-bottom or a red-cyan anaglyph (INTEGRATION.md).
 """
 from __future__ import annotations
 
 import os
+import struct
 import sys
 import threading
 import time
@@ -25,6 +29,8 @@ from concurrent.futures import ThreadPoolExecutor
 from pathlib import Path
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+
+from vsc_b200.stereo_core import LAYOUTS  # noqa: E402
 
 GPU_ERROR_EXIT_CODE = 100      # reference: sbs_generator.py:41
 
@@ -53,7 +59,42 @@ def build_parser() -> ArgumentParser:
     p.add_argument('--raw-sink', default=None, metavar='PATH',
                    help="hand the SBS frames to an encoder instead of writing sbs_*.png: raw rgb24, in clip order, into PATH "
                         "(a file or FIFO; '-' = stdout); geometry in PATH.json.  Processes every frame pair (no resume)")
+    p.add_argument('--layout', choices=LAYOUTS, default=None,
+                   help="output frame layout (default: config.json \"sbs_layout\", else sbs): sbs [H,2W], half-sbs [H,W], "
+                        "tb [2H,W], half-tb [H,W], anaglyph [H,W] (red-cyan)")
     return p
+
+
+def png_size(path):
+    """(height, width) from a PNG's IHDR chunk (bytes 16-24) without decoding it; None if the file is no PNG."""
+    try:
+        with open(path, 'rb') as f:
+            head = f.read(24)
+    except OSError:
+        return None
+    if len(head) < 24 or head[:8] != b'\x89PNG\r\n\x1a\n' or head[12:16] != b'IHDR':
+        return None
+    w, h = struct.unpack('>II', head[16:24])
+    return h, w
+
+
+def layout_refusal(output_dir: Path, frame_path, layout: str):
+    """Why `layout` cannot continue this clip, or None.  The layout must take the frame size, and on a resume the
+    outputs already written must have the size this layout gives (one clip with mixed frame sizes breaks the encode)."""
+    from vsc_b200.stereo_core import output_shape
+    size = png_size(frame_path)
+    if size is None:
+        return None
+    try:
+        want = output_shape(layout, *size)[:2]
+    except ValueError as e:
+        return str(e)
+    existing = sorted(output_dir.glob('sbs_*.png'))
+    have = png_size(existing[0]) if existing else None
+    if have is not None and have != want:
+        return (f"{existing[0].name} is {have[1]}x{have[0]}, but layout '{layout}' makes {want[1]}x{want[0]} frames of this "
+                f"clip: continue with the layout the existing outputs were written in, or move them away")
+    return None
 
 
 def _decode_into(item, gen, slot, index, expected):
@@ -84,8 +125,22 @@ def _decode_into(item, gen, slot, index, expected):
         return 'error', str(e)
 
 
+def open_raw_sink(path: str, pairs, layout: str):
+    """RawFrameSink for `pairs` in clip order; frame geometry (and the JSON side-car) from the first frame and the
+    layout.  OSError when the first frame cannot be read, ValueError when the layout cannot take its size."""
+    import cv2
+    from vsc_b200.sharder import RawFrameSink
+    from vsc_b200.stereo_core import output_shape
+    probe = cv2.imread(str(pairs[0][0]), cv2.IMREAD_COLOR)
+    if probe is None:
+        raise OSError(f'cannot read {pairs[0][0]}')
+    oh, ow, _ = output_shape(layout, probe.shape[0], probe.shape[1])
+    return RawFrameSink(path, len(pairs), oh, ow, frame_numbers=[p[2] for p in pairs])
+
+
 def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int, io_threads: int, free_space_mode: str,
-                  no_interactive: bool, progress=None, sink=None, sink_index=None, group: int = 4, gen=None) -> int:
+                  no_interactive: bool, progress=None, sink=None, sink_index=None, group: int = 4, gen=None,
+                  layout: str = 'sbs') -> int:
     """Run `pairs` [(frame_path, depth_path, frame_num)] through one GPU.  Returns frames written.
 
     The pipeline the benchmark times: `slots` frame slots of `group` frames each.  A slot is filled by the loader
@@ -93,7 +148,7 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
     stream, one hole-filling launch for the group) and harvested with vsc_wait_any; finished frames go to the saver
     pool (bounded backlog) and become visible in frame order through the InOrderPublisher.
     With `sink` (a RawFrameSink shared by all GPUs of the process) frames go to it at position
-    `sink_index[frame_num]` instead of into sbs_<n>.png."""
+    `sink_index[frame_num]` instead of into sbs_<n>.png.  `layout` is the output layout of a generator made here."""
     import cv2
     import numpy as np
     from vsc_b200 import StereoGenerator
@@ -101,7 +156,7 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
 
     own_gen = gen is None         # a caller may pass a warm generator (n_slots >= slots, group_size >= group) and keep it
     if own_gen:
-        gen = StereoGenerator(f'cuda:{device_index}', n_slots=slots, group_size=group)
+        gen = StereoGenerator(f'cuda:{device_index}', n_slots=slots, group_size=group, layout=layout)
     loaders = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='load')
     savers = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='save')
     backlog = threading.BoundedSemaphore(max(2 * io_threads, group))     # frames waiting for / inside the savers
@@ -249,11 +304,12 @@ def main(argv=None) -> int:
         print(f'ERROR: Workflow directory not found: {args.workflow_path}')
         return 0
     ConfigError, get_path, load_config = _load_config_api()
+    from vsc_b200.workflow import LayoutError, config_layout
     try:
         config = load_config(args.workflow_path)
     except ConfigError as e:
         print(f'ERROR: {e}')
-        return 0
+        return 2 if isinstance(e, LayoutError) else 0
     frames_dir = get_path(args.workflow_path, config, 'frames')
     depth_dir = get_path(args.workflow_path, config, 'depth_maps')
     output_dir = get_path(args.workflow_path, config, 'sbs')
@@ -266,6 +322,11 @@ def main(argv=None) -> int:
     output_dir.mkdir(parents=True, exist_ok=True)
     if args.cpu:
         print('ERROR: --cpu is not supported: the B200 SBS path has no CPU fallback (use the reference implementation).')
+        return 2
+    try:
+        layout = args.layout or config_layout(config)
+    except LayoutError as e:
+        print(f'ERROR: {e}')
         return 2
 
     from vsc_b200 import StereoParams
@@ -289,6 +350,10 @@ def main(argv=None) -> int:
         if rank == 0:
             print('All frames already processed.')
         return 0
+    why = layout_refusal(output_dir, pairs[0][0], layout) if not args.raw_sink else None
+    if why:
+        print(f'ERROR: {why}')
+        return 2
 
     import torch
     if not torch.cuda.is_available():
@@ -300,7 +365,7 @@ def main(argv=None) -> int:
         print(f'Using GPU: {torch.cuda.get_device_name(0)} x{world if world > 1 else (args.gpus or ngpu)}')
         print(f'Parameters: disparity={params.max_disparity}, convergence={params.convergence}, '
               f'super_sampling={params.super_sampling}, edge_softness={params.edge_softness}, '
-              f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}')
+              f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}, layout={layout}')
 
     finals = [str(output_dir / f'sbs_{p[2]}.png') for p in pairs]
 
@@ -314,13 +379,14 @@ def main(argv=None) -> int:
         if world > 1:
             print('ERROR: --raw-sink needs all GPUs in one process (use --gpus N, not torchrun)')
             return 2
-        import cv2
-        from vsc_b200.sharder import RawFrameSink
-        probe = cv2.imread(str(pairs[0][0]), cv2.IMREAD_COLOR)
-        if probe is None:
-            print(f'ERROR: cannot read {pairs[0][0]}')
+        try:
+            sink = open_raw_sink(args.raw_sink, pairs, layout)
+        except OSError as e:
+            print(f'ERROR: {e}')
             return 0
-        sink = RawFrameSink(args.raw_sink, len(pairs), probe.shape[0], 2 * probe.shape[1], frame_numbers=[p[2] for p in pairs])
+        except ValueError as e:         # the layout cannot take the frame size
+            print(f'ERROR: {e}')
+            return 2
         sink_index = {p[2]: i for i, p in enumerate(pairs)}
     t0 = time.time()
     done = [0]
@@ -344,7 +410,7 @@ def main(argv=None) -> int:
             if t:
                 t.start()
             n = process_shard(mine, output_dir, params, local_rank, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                              group=args.group)
+                              group=args.group, layout=layout)
             barrier()
             if t:
                 pub.stop()
@@ -359,7 +425,7 @@ def main(argv=None) -> int:
             t.start()
             if g == 1:
                 n = process_shard(pairs, output_dir, params, 0, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                                  sink, sink_index, args.group)
+                                  sink, sink_index, args.group, layout=layout)
             else:
                 # one worker thread per GPU; each owns a StereoGenerator (its own CUDA context state, streams, pinned ring)
                 results = [0] * g
@@ -368,7 +434,8 @@ def main(argv=None) -> int:
                 def work(k):
                     try:
                         results[k] = process_shard(shard_items(pairs, g, k), output_dir, params, k, args.slots, args.io_threads,
-                                                   free_space_mode, args.no_interactive, progress, sink, sink_index, args.group)
+                                                   free_space_mode, args.no_interactive, progress, sink, sink_index, args.group,
+                                                   layout=layout)
                     except BaseException as e:   # noqa: BLE001
                         errors.append(e)
                 ths = [threading.Thread(target=work, args=(k,)) for k in range(g)]

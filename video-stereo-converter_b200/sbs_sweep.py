@@ -11,7 +11,8 @@ renders the cartesian product of the given values (every other parameter from co
 `sweep_<i>.png` plus `sweep.json` (parameters, milliseconds, refusals) into `--out`, through the same
 `StereoGenerator` the batch driver uses.  Parameter names, ranges and step sizes are the tester's sliders
 (sbs_tester.py:356-362); a combination whose convergence crop is invalid is recorded as refused, like the
-tester's red status line.
+tester's red status line.  `--layout anaglyph` renders red-cyan previews, which show the depth effect of
+`max_disparity` and `convergence` on any screen with a pair of red-cyan glasses.
 """
 from __future__ import annotations
 
@@ -24,6 +25,8 @@ from argparse import ArgumentParser
 from pathlib import Path
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+
+from vsc_b200.stereo_core import LAYOUTS  # noqa: E402
 
 # slider ranges of the reference's tester: name -> (from, to, step)   (sbs_tester.py:356-362)
 SLIDERS = {
@@ -83,11 +86,14 @@ def main(argv=None) -> int:
     ap.add_argument('--out', type=Path, default=None, help='output directory (default: <workflow>/sweep)')
     ap.add_argument('--slots', type=int, default=4, help='frames in flight')
     ap.add_argument('--no-images', action='store_true', help='only write sweep.json (timings, refusals)')
+    ap.add_argument('--layout', choices=LAYOUTS, default=None,
+                    help='output layout of the previews (default: config.json "sbs_layout", else sbs)')
     args = ap.parse_args(argv)
 
-    from vsc_b200.workflow import ConfigError, find_frame_pairs, get_path, load_config
+    from vsc_b200.workflow import ConfigError, config_layout, find_frame_pairs, get_path, load_config
     try:
         config = load_config(args.workflow_path)
+        layout = args.layout or config_layout(config)
     except ConfigError as e:
         print(f'ERROR: {e}')
         return 2
@@ -111,7 +117,7 @@ def main(argv=None) -> int:
     rgb, depth = load_image_pair(frame_path, depth_path)
     out_dir = args.out or (args.workflow_path / 'sweep')
     out_dir.mkdir(parents=True, exist_ok=True)
-    gen = StereoGenerator('cuda:0', n_slots=max(1, args.slots))
+    gen = StereoGenerator('cuda:0', n_slots=max(1, args.slots), layout=layout)
     results = [None] * len(combos)
     t0 = time.time()
     inflight, free = [], list(range(gen.n_slots))
@@ -143,7 +149,8 @@ def main(argv=None) -> int:
     dt = time.time() - t0
     ok = [r for r in results if r['refused'] is None]
     with open(out_dir / 'sweep.json', 'w') as f:
-        json.dump({'frame': int(frame_num), 'shape': list(rgb.shape), 'swept': args.param, 'seconds': round(dt, 3), 'results': results}, f, indent=1)
+        json.dump({'frame': int(frame_num), 'shape': list(rgb.shape), 'layout': layout, 'swept': args.param, 'seconds': round(dt, 3),
+                   'results': results}, f, indent=1)
     print(f'{len(ok)} of {len(combos)} parameter sets rendered in {dt:.2f} s ({len(ok) / max(dt, 1e-9):.1f} previews/s), '
           f'{len(combos) - len(ok)} refused; results in {out_dir}')
     return 0

@@ -6,7 +6,9 @@ sm_100a CUDA kernels behind the C ABI of include/vsc_b200.h.  There is no CPU pa
 `StereoGenerator('cpu')` raises, and a missing CUDA library raises on import of `_lib`.
 
 Additions that the reference does not have (used by the frame loop in sbs_generator.py):
-`StereoGenerator.submit/collect` (asynchronous, pinned, multi-slot) and `process_batch`.
+`StereoGenerator.submit/collect` (asynchronous, pinned, multi-slot) and `process_batch`, and output layouts
+(`StereoGenerator(..., layout='half-sbs')`, `LAYOUTS`, `output_shape`): every output path then returns frames of
+`output_shape(layout, h, w)` instead of the side-by-side [h, 2w, 3].
 """
 from __future__ import annotations
 
@@ -40,6 +42,28 @@ class StereoParams:
     artifact_smoothing: float = 1.0
     depth_gamma: float = 0.2
     sharpen: float = 14.0
+
+
+# output layouts (include/vsc_b200.h VSC_LAYOUT_*): name -> C enum.  'sbs' is the reference's output.
+LAYOUTS = ('sbs', 'half-sbs', 'tb', 'half-tb', 'anaglyph')
+
+
+def layout_code(layout: str) -> int:
+    """C enum of a layout name; ValueError for anything else."""
+    if layout not in LAYOUTS:
+        raise ValueError(f'unknown output layout {layout!r} (one of {", ".join(LAYOUTS)})')
+    return LAYOUTS.index(layout)
+
+
+def output_shape(layout: str, h: int, w: int) -> Tuple[int, int, int]:
+    """Shape (rows, cols, 3) of the frame `layout` makes of an h x w input (the library's vsc_layout_shape).
+    ValueError for an unknown layout or an odd side that a half layout halves."""
+    code = layout_code(layout)
+    oh, ow = C.c_int(), C.c_int()
+    rc = _lib.load().vsc_layout_shape(code, int(h), int(w), C.byref(oh), C.byref(ow))
+    if rc != _lib.VSC_OK:
+        raise ValueError((_lib.load().vsc_last_error() or b'').decode('utf-8', 'replace'))
+    return oh.value, ow.value, 3
 
 
 # ------------------------------------------------------------------------------------------------
@@ -158,13 +182,17 @@ class StereoGenerator:
 
     `process_frame(rgb, depth, params)` keeps the reference's numpy-in / numpy-out contract.
     `n_slots` frames can be in flight through `submit` / `collect` for the driver loop.
+    `layout` (one of LAYOUTS, default the reference's 'sbs') sets the shape of every frame this generator returns.
     """
     _DEFAULT_PARAMS = StereoParams()
 
-    def __init__(self, device: str, n_slots: int = 1, group_size: int = 1) -> None:
+    def __init__(self, device: str, n_slots: int = 1, group_size: int = 1, layout: str = 'sbs') -> None:
         self.device = device
+        code = layout_code(layout)
         self._ctx = _lib.Context(_parse_device(device), n_slots, group_size)
         self._lib = _lib.load()
+        _lib.check(self._lib.vsc_set_layout(self._ctx.handle, code))
+        self.layout = layout
         self.n_slots, self.group_size = n_slots, group_size
         self._pending = [None] * n_slots        # per slot: number of frames in flight
         # pinned staging per (slot, frame index within the slot's group): (key, rgb, depth, out) PinnedBuffers
@@ -172,11 +200,12 @@ class StereoGenerator:
 
     # -- reference API ---------------------------------------------------------------------------
     def process_frame(self, rgb: np.ndarray, depth: np.ndarray, params: StereoParams | None = None) -> np.ndarray:
-        """Process a single frame to a side-by-side stereo image (left | right), uint8 [H, 2W, 3]."""
+        """Process a single frame to a side-by-side stereo image (left | right), uint8 [H, 2W, 3]
+        (with another layout: uint8 of output_shape(layout, H, W))."""
         p = params or self._DEFAULT_PARAMS
         rgb_c, depth_c, code = self._check_inputs(rgb, depth)
         h, w = rgb_c.shape[:2]
-        out = np.empty((h, 2 * w, 3), np.uint8)
+        out = np.empty(self.output_shape(h, w), np.uint8)
         _lib.check(self._lib.vsc_process_frame(self._ctx.handle, _lib.ptr(rgb_c), _lib.ptr(depth_c), code, h, w,
                                                C.byref(_lib.make_params(p)), _lib.ptr(out)))
         return out
@@ -185,6 +214,7 @@ class StereoGenerator:
     def pinned_inputs(self, slot: int, h: int, w: int, depth_dtype=np.uint8, index: int = 0):
         """Page-locked (rgb[h,w,3], depth[h,w]) arrays of frame `index` of `slot` for a loader to decode into."""
         key = (int(h), int(w), np.dtype(depth_dtype).str)
+        self.output_shape(h, w)             # a size the layout cannot take is refused before any buffer changes
         pin = self._pinned[slot][index]
         if pin is None or pin[0] != key:
             if self._pending[slot] is not None:
@@ -193,7 +223,7 @@ class StereoGenerator:
                 for b in pin[1:]:
                     b.free()
             pin = (key, _lib.PinnedBuffer((h, w, 3), np.uint8), _lib.PinnedBuffer((h, w), depth_dtype),
-                   _lib.PinnedBuffer((h, 2 * w, 3), np.uint8))
+                   _lib.PinnedBuffer(self.output_shape(h, w), np.uint8))
             self._pinned[slot][index] = pin
         return pin[1].array, pin[2].array
 
@@ -262,7 +292,7 @@ class StereoGenerator:
         self.submit_pinned(slot, params, len(frames))
 
     def collect(self, slot: int, copy: bool = True):
-        """Wait for the slot's submission.  Returns the SBS frame (a list of frames if more than one was
+        """Wait for the slot's submission.  Returns the output frame (a list of frames if more than one was
         submitted).  copy=True returns fresh arrays the caller owns (the reference hands its result to another
         thread, sbs_generator.py:325, so it must not alias a reused buffer); copy=False returns the pinned
         outputs, valid until the slot is submitted again."""
@@ -281,7 +311,8 @@ class StereoGenerator:
 
     def submit_device(self, slot: int, d_rgb: int, d_depth: int, depth_dtype, h: int, w: int, d_out: int,
                       params: StereoParams | None = None) -> None:
-        """Device-resident variant: raw device pointers (e.g. torch tensor .data_ptr()), no copies."""
+        """Device-resident variant: raw device pointers (e.g. torch tensor .data_ptr()), no copies.  d_out must hold
+        output_shape(h, w) uint8."""
         p = params or self._DEFAULT_PARAMS
         _lib.check(self._lib.vsc_submit_device(self._ctx.handle, slot, C.c_void_p(d_rgb), C.c_void_p(d_depth),
                                                _lib.depth_code(depth_dtype), h, w, C.byref(_lib.make_params(p)),
@@ -410,7 +441,26 @@ class StereoGenerator:
         self._pinned = [[None] * self.group_size for _ in range(self.n_slots)]
         self._ctx.close()
 
+    def set_layout(self, layout: str) -> None:
+        """Switch the output layout of frames submitted from now on.  Every slot must be collected: the pinned output
+        buffers of the old shape are released (pinned_inputs allocates them again)."""
+        code = layout_code(layout)
+        if any(x is not None for x in self._pending):
+            raise RuntimeError('collect every slot before changing the layout')
+        _lib.check(self._lib.vsc_set_layout(self._ctx.handle, code))
+        self.layout = layout
+        for row in self._pinned:
+            for i, pin in enumerate(row):
+                if pin is not None:
+                    for b in pin[1:]:
+                        b.free()
+                    row[i] = None
+
     # -- helpers -----------------------------------------------------------------------------------
+    def output_shape(self, h: int, w: int) -> Tuple[int, int, int]:
+        """Shape of the frames this generator returns for h x w inputs."""
+        return output_shape(self.layout, h, w)
+
     @staticmethod
     def _check_inputs(rgb: np.ndarray, depth: np.ndarray):
         if rgb.ndim != 3 or rgb.shape[2] != 3:

@@ -4,6 +4,10 @@ The reference's helper/config_manager.py (load_config :267, get_path :342, the `
 :43-54) stays the owner of the format; this module reads the same file with the same rules for the
 keys this stage needs, so that sbs_generator.py runs both inside the reference tree (where
 `helper.config_manager` is importable and preferred) and standalone.
+
+One key is this implementation's own: the optional top-level "sbs_layout" (output layout of the SBS stage, one of
+stereo_core.LAYOUTS, default "sbs").  It sits at the top level because the reference's validator accepts extra
+top-level keys while the reference builds StereoParams from the whole `stereo` block.
 """
 from __future__ import annotations
 
@@ -13,10 +17,24 @@ from typing import Dict
 
 STEREO_KEYS = ('max_disparity', 'convergence', 'super_sampling', 'edge_softness', 'artifact_smoothing', 'depth_gamma', 'sharpen')
 DIR_KEYS = ('frames', 'depth_maps', 'sbs')
+LAYOUT_KEY = 'sbs_layout'
 
 
 class ConfigError(Exception):
     """Raised when config.json is missing or fails validation (reference: config_manager.py:78)."""
+
+
+class LayoutError(ConfigError):
+    """The optional "sbs_layout" key holds something other than a layout name."""
+
+
+def config_layout(cfg: Dict) -> str:
+    """The output layout a config asks for: top-level "sbs_layout", default 'sbs'."""
+    from .stereo_core import LAYOUTS
+    v = cfg.get(LAYOUT_KEY, 'sbs')
+    if v not in LAYOUTS:
+        raise LayoutError(f"Invalid '{LAYOUT_KEY}' {v!r} (expected one of {', '.join(LAYOUTS)})")
+    return v
 
 
 def load_config(workflow_path) -> Dict:
@@ -39,6 +57,7 @@ def load_config(workflow_path) -> Dict:
         # ints are accepted for floats (config_manager.py:114); bools are not numbers here
         if isinstance(v, bool) or not isinstance(v, (int, float)):
             raise ConfigError(f"Missing or invalid 'stereo.{k}' (expected float)")
+    config_layout(cfg)
     return cfg
 
 
