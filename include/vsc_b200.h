@@ -140,6 +140,29 @@ int vsc_layout_shape(int layout, int height, int width, int *out_h, int *out_w);
  * it is the store epilogue of the back-end kernel.  vsc_stage_backend always writes SBS. */
 int vsc_set_layout(vsc_ctx *ctx, int layout);
 
+/* -------- output pixel formats (no reference counterpart) -------------------------------------- */
+/* A pixel format is a fixed integer function of the final u8 RGB frame of the chosen layout (oh x ow,
+ * vsc_layout_shape), so it inherits that frame's exactness.  All int32, no floats, no clamps; S = sum over a 2x2 block
+ * (centre-sited chroma), cc = cu for Cb and cv for Cr, limited ("tv") range:
+ *   Y8  = (cy.(r,g,b) + (16<<20) + (1<<19)) >> 20        C8  = (cc.(Sr,Sg,Sb) + (128<<22) + (1<<21)) >> 22
+ *   Y10 = (cy.(r,g,b) + (16<<20) + (1<<17)) >> 18        C10 = (cc.(Sr,Sg,Sb) + (128<<22) + (1<<19)) >> 20
+ *   BT709: cy = 191455 644068 65019   cu = -105533 -355018 460551   cv = 460551 -418321 -42230   (Kr .2126, Kb .0722, Q20)
+ *   BT601: cy = 269484 528482 102760  cu = -155188 -305135 460324   cv = 460324 -385875 -74448   (OpenCV's RGB2YUV_I420)
+ *   RGB24        [oh][ow][3] bytes (the default)
+ *   YUV420P      I420: Y [oh][ow], U [oh/2][ow/2], V [oh/2][ow/2], bytes                      (oh*ow*3/2 bytes)
+ *   YUV420P10LE  the same planes as little-endian uint16, the value in the low 10 bits    (oh*ow*3 bytes)
+ * The YUV formats take an even H and W only, and also W % 4 == 0 with HALF_SBS and H % 4 == 0 with HALF_TB (each eye
+ * then starts on an even coordinate of the output frame). */
+enum { VSC_PIXFMT_RGB24 = 0, VSC_PIXFMT_YUV420P = 1, VSC_PIXFMT_YUV420P10LE = 2 };
+enum { VSC_MATRIX_BT709 = 0, VSC_MATRIX_BT601 = 1 };
+/* host only: bytes of one output frame of an H x W input in (layout, pixfmt); VSC_E_INVALID for an unknown layout or
+ * format or a size they cannot take */
+int vsc_output_size(int layout, int pixfmt, int height, int width, size_t *bytes);
+/* pixel format and YUV matrix of frames submitted to ctx from now on (like vsc_set_layout: frames in flight keep
+ * theirs).  Default VSC_PIXFMT_RGB24 / VSC_MATRIX_BT709.  out buffers must hold vsc_output_size bytes.  No kernel
+ * launch is added: the conversion is the store epilogue of the back-end kernel.  vsc_stage_backend always writes RGB24. */
+int vsc_set_pixfmt(vsc_ctx *ctx, int pixfmt, int matrix);
+
 /* -------- stage-level entry points for per-stage parity tests (host buffers, synchronous) --- */
 /* cv2.resize(src,(dst_w,H),INTER_LANCZOS4) (stereo_core.py:253-254); channels 1 or 3 for u8 */
 int vsc_stage_lanczos(vsc_ctx *ctx, const void *src, int dtype, int channels, int height, int width,

@@ -262,6 +262,7 @@ struct Slot {
     const uint8_t* l_rgb = nullptr; const void* l_depth = nullptr; uint8_t* l_out = nullptr;
     int l_dtype = 0, l_H = 0, l_W = 0; vsc_params l_p; uint8_t* l_host_out = nullptr; size_t l_out_bytes = 0;
     int l_layout = VSC_LAYOUT_SBS;       // output layout of the frame in this slot (fixed at submission)
+    int l_pixfmt = VSC_PIXFMT_RGB24, l_matrix = VSC_MATRIX_BT709;   // its pixel format and YUV matrix (the same)
     int launches = 0;
     float last_ms = 0.f;
     bool done = false;                   // leader only: the stream has run past the submission (set by a host callback)
@@ -278,6 +279,8 @@ struct vsc_ctx {
     int group_size = 1;                  // frames that share one stream and one hole-filling launch
     bool profiling = false;
     int layout = VSC_LAYOUT_SBS;         // output layout of frames submitted from now on (vsc_set_layout)
+    int pixfmt = VSC_PIXFMT_RGB24;       // pixel format and YUV matrix of frames submitted from now on (vsc_set_pixfmt)
+    int matrix = VSC_MATRIX_BT709;
     cudaStream_t tstream = nullptr;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     std::vector<cudaEvent_t> tslot;
@@ -345,12 +348,19 @@ static int upload_constants(vsc_ctx* ctx) {
     return VSC_OK;
 }
 
+template <int K, int P>
+static int backend_attrs(int smem) {
+    const void* f[] = {(const void*)backend_kernel<K, VSC_LAYOUT_SBS, P>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_SBS, P>,
+                       (const void*)backend_kernel<K, VSC_LAYOUT_TB, P>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_TB, P>,
+                       (const void*)backend_kernel<K, VSC_LAYOUT_ANAGLYPH, P>};
+    for (const void* k : f) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    return VSC_OK;
+}
 template <int K>
 static int backend_attrs(int smem) {
-    const void* f[] = {(const void*)backend_kernel<K, VSC_LAYOUT_SBS>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_SBS>,
-                       (const void*)backend_kernel<K, VSC_LAYOUT_TB>, (const void*)backend_kernel<K, VSC_LAYOUT_HALF_TB>,
-                       (const void*)backend_kernel<K, VSC_LAYOUT_ANAGLYPH>};
-    for (const void* k : f) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    int rc;
+    if ((rc = backend_attrs<K, VSC_PIXFMT_RGB24>(smem)) || (rc = backend_attrs<K, VSC_PIXFMT_YUV420P>(smem)) ||
+        (rc = backend_attrs<K, VSC_PIXFMT_YUV420P10LE>(smem))) return rc;
     return VSC_OK;
 }
 static int set_smem_attrs() {
@@ -702,20 +712,35 @@ static int run_telea(vsc_ctx* ctx, Slot& s, int Hs, int Ws, const ViewSpec* vs, 
 #endif
     return VSC_OK;
 }
-template <int K>
-static void launch_backend(int layout, dim3 grid, size_t smem, cudaStream_t st, const BackendArgs& a) {
-    switch (layout) {
-        case VSC_LAYOUT_HALF_SBS: backend_kernel<K, VSC_LAYOUT_HALF_SBS><<<grid, kThreads, smem, st>>>(a); break;
-        case VSC_LAYOUT_TB: backend_kernel<K, VSC_LAYOUT_TB><<<grid, kThreads, smem, st>>>(a); break;
-        case VSC_LAYOUT_HALF_TB: backend_kernel<K, VSC_LAYOUT_HALF_TB><<<grid, kThreads, smem, st>>>(a); break;
-        case VSC_LAYOUT_ANAGLYPH: grid.z = 1; backend_kernel<K, VSC_LAYOUT_ANAGLYPH><<<grid, kThreads, smem, st>>>(a); break;
-        default: backend_kernel<K, VSC_LAYOUT_SBS><<<grid, kThreads, smem, st>>>(a); break;
+template <int K, int L>
+static void launch_backend(int pixfmt, dim3 grid, size_t smem, cudaStream_t st, const BackendArgs& a) {
+    switch (pixfmt) {
+        case VSC_PIXFMT_YUV420P: backend_kernel<K, L, VSC_PIXFMT_YUV420P><<<grid, kThreads, smem, st>>>(a); break;
+        case VSC_PIXFMT_YUV420P10LE: backend_kernel<K, L, VSC_PIXFMT_YUV420P10LE><<<grid, kThreads, smem, st>>>(a); break;
+        default: backend_kernel<K, L, VSC_PIXFMT_RGB24><<<grid, kThreads, smem, st>>>(a); break;
     }
 }
-// d_out holds the frame in `layout` (vsc_layout_shape; the caller has checked that the layout takes H x W)
+template <int K>
+static void launch_backend(int layout, int pixfmt, dim3 grid, size_t smem, cudaStream_t st, const BackendArgs& a) {
+    switch (layout) {
+        case VSC_LAYOUT_HALF_SBS: launch_backend<K, VSC_LAYOUT_HALF_SBS>(pixfmt, grid, smem, st, a); break;
+        case VSC_LAYOUT_TB: launch_backend<K, VSC_LAYOUT_TB>(pixfmt, grid, smem, st, a); break;
+        case VSC_LAYOUT_HALF_TB: launch_backend<K, VSC_LAYOUT_HALF_TB>(pixfmt, grid, smem, st, a); break;
+        case VSC_LAYOUT_ANAGLYPH: grid.z = 1; launch_backend<K, VSC_LAYOUT_ANAGLYPH>(pixfmt, grid, smem, st, a); break;
+        default: launch_backend<K, VSC_LAYOUT_SBS>(pixfmt, grid, smem, st, a); break;
+    }
+}
+// the YUV matrices of include/vsc_b200.h: rows cy, cu, cv in Q20 (BT.709 from Kr = 0.2126, Kb = 0.0722; BT.601 is
+// OpenCV's RGB2YUV_I420 table)
+static const int kYuvMatrix[2][9] = {
+    {191455, 644068, 65019, -105533, -355018, 460551, 460551, -418321, -42230},
+    {269484, 528482, 102760, -155188, -305135, 460324, 460324, -385875, -74448},
+};
+// d_out holds the frame in `layout` and `pixfmt` (vsc_output_size; the caller has checked that they take H x W)
 static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4* v0, const uchar4* v1, uint8_t* d_out,
-                       int layout) {
+                       int layout, int pixfmt = VSC_PIXFMT_RGB24, int matrix = VSC_MATRIX_BT709) {
     BackendArgs a;
+    memcpy(a.yuv, kYuvMatrix[matrix], sizeof a.yuv);
     a.view[0] = v0; a.view[1] = v1; a.out = d_out;
     a.H = g.height; a.W = g.width; a.Hs = g.ss_h; a.Ws = g.ss_w;
     a.crop[0] = g.left_crop; a.crop[1] = g.right_crop; a.cw = g.crop_w;
@@ -734,10 +759,10 @@ static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4*
     dim3 grid((g.width + BE_OX - 1) / BE_OX, (g.height + BE_OY - 1) / BE_OY, 2);
     prof_begin(s, "backend_kernel");
     switch (K) {       // the anaglyph runs both eyes in one CTA (grid.z = 1)
-        case 2: launch_backend<2>(layout, grid, smem, s.stream, a); break;
-        case 3: launch_backend<3>(layout, grid, smem, s.stream, a); break;
-        case 4: launch_backend<4>(layout, grid, smem, s.stream, a); break;
-        default: launch_backend<0>(layout, grid, smem, s.stream, a); break;
+        case 2: launch_backend<2>(layout, pixfmt, grid, smem, s.stream, a); break;
+        case 3: launch_backend<3>(layout, pixfmt, grid, smem, s.stream, a); break;
+        case 4: launch_backend<4>(layout, pixfmt, grid, smem, s.stream, a); break;
+        default: launch_backend<0>(layout, pixfmt, grid, smem, s.stream, a); break;
     }
     KCHECK(s);
     return VSC_OK;
@@ -805,7 +830,8 @@ static int enqueue_group(vsc_ctx* ctx, Slot* fr, int n, int dtype, const vsc_geo
     int rc = run_telea(ctx, lead, g.ss_h, g.ss_w, vs, 2 * n);
     if (rc) return rc;
     for (int i = 0; i < n; i++)
-        if ((rc = run_backend(fr[i], g, p.sharpen, cur[2 * i], cur[2 * i + 1], fr[i].l_out, fr[i].l_layout))) return rc;
+        if ((rc = run_backend(fr[i], g, p.sharpen, cur[2 * i], cur[2 * i + 1], fr[i].l_out, fr[i].l_layout,
+                                  fr[i].l_pixfmt, fr[i].l_matrix))) return rc;
     CU(cudaEventRecord(lead.ev1, lead.stream));
     for (int i = 0; i < n; i++)
         CU(cudaMemcpyAsync(fr[i].h_scalars, fr[i].scalars.p, sizeof(FrameScalars), cudaMemcpyDeviceToHost, lead.stream));
@@ -836,15 +862,15 @@ static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const
     vsc_geom g;
     int rc;
     if ((rc = vsc_geometry(H, W, p, &g))) return rc;
-    const int layout = ctx->layout;
-    int oh, ow;
-    if ((rc = vsc_layout_shape(layout, H, W, &oh, &ow))) return rc;
+    const int layout = ctx->layout, pixfmt = ctx->pixfmt, matrix = ctx->matrix;
+    size_t nout;
+    if ((rc = vsc_output_size(layout, pixfmt, H, W, &nout))) return rc;
     CU(cudaSetDevice(ctx->device));
-    const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype), nout = (size_t)oh * ow * 3;
+    const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype);
     for (int i = 0; i < n; i++) {
         Slot& s = fr[i];
         s.l_rgb = rgb[i]; s.l_depth = depth[i]; s.l_out = out[i]; s.l_host_out = nullptr; s.l_out_bytes = nout;
-        s.l_layout = layout;
+        s.l_layout = layout; s.l_pixfmt = pixfmt; s.l_matrix = matrix;
         if (!device_io) {
             if (s.in_rgb.ensure(nrgb) || s.in_depth.ensure(ndepth) || s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
             CU(cudaMemcpyAsync(s.in_rgb.p, rgb[i], nrgb, cudaMemcpyHostToDevice, lead.stream));
@@ -1001,6 +1027,31 @@ extern "C" int vsc_set_layout(vsc_ctx* ctx, int layout) {
     if (!ctx) return fail(VSC_E_INVALID, "null context");
     if (layout < VSC_LAYOUT_SBS || layout > VSC_LAYOUT_ANAGLYPH) return fail(VSC_E_INVALID, "unknown output layout %d", layout);
     ctx->layout = layout;
+    return VSC_OK;
+}
+extern "C" int vsc_output_size(int layout, int pixfmt, int H, int W, size_t* bytes) {
+    if (!bytes) return fail(VSC_E_INVALID, "null argument");
+    int oh, ow, rc;
+    if ((rc = vsc_layout_shape(layout, H, W, &oh, &ow))) return rc;
+    const size_t n = (size_t)oh * ow;
+    switch (pixfmt) {
+        case VSC_PIXFMT_RGB24: *bytes = n * 3; return VSC_OK;
+        case VSC_PIXFMT_YUV420P: case VSC_PIXFMT_YUV420P10LE: break;
+        default: return fail(VSC_E_INVALID, "unknown pixel format %d", pixfmt);
+    }
+    // 4:2:0 needs whole 2x2 blocks, and each eye must start on an even coordinate of the output frame
+    if (H % 2 || W % 2) return fail(VSC_E_INVALID, "yuv420 needs an even frame size: %dx%d", W, H);
+    if (layout == VSC_LAYOUT_HALF_SBS && W % 4) return fail(VSC_E_INVALID, "yuv420 with half-sbs needs a width divisible by 4: %d", W);
+    if (layout == VSC_LAYOUT_HALF_TB && H % 4) return fail(VSC_E_INVALID, "yuv420 with half-tb needs a height divisible by 4: %d", H);
+    *bytes = pixfmt == VSC_PIXFMT_YUV420P ? n * 3 / 2 : n * 3;
+    return VSC_OK;
+}
+extern "C" int vsc_set_pixfmt(vsc_ctx* ctx, int pixfmt, int matrix) {
+    if (!ctx) return fail(VSC_E_INVALID, "null context");
+    if (pixfmt < VSC_PIXFMT_RGB24 || pixfmt > VSC_PIXFMT_YUV420P10LE) return fail(VSC_E_INVALID, "unknown pixel format %d", pixfmt);
+    if (matrix < VSC_MATRIX_BT709 || matrix > VSC_MATRIX_BT601) return fail(VSC_E_INVALID, "unknown yuv matrix %d", matrix);
+    ctx->pixfmt = pixfmt;
+    ctx->matrix = matrix;
     return VSC_OK;
 }
 

@@ -16,6 +16,8 @@ There is no CPU path: `--cpu` is refused.
 
 `--layout` (or the top-level config.json key "sbs_layout") picks the output frame layout: the reference's full-width
 side-by-side (default), half side-by-side, top-bottom, half top-bottom or a red-cyan anaglyph (INTEGRATION.md).
+`--pixfmt` / `--matrix` (or the top-level keys "sbs_pixfmt" / "sbs_matrix") hand the raw sink encoder-ready YUV 4:2:0
+(yuv420p, yuv420p10le; BT.709 or BT.601, limited range) instead of rgb24; a YUV format needs `--raw-sink`.
 """
 from __future__ import annotations
 
@@ -30,7 +32,7 @@ from pathlib import Path
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
-from vsc_b200.stereo_core import LAYOUTS  # noqa: E402
+from vsc_b200.stereo_core import LAYOUTS, MATRICES, PIXFMTS  # noqa: E402
 
 GPU_ERROR_EXIT_CODE = 100      # reference: sbs_generator.py:41
 
@@ -57,11 +59,16 @@ def build_parser() -> ArgumentParser:
     p.add_argument('--group', type=int, default=4, help='frames per slot submission (they share one hole-filling launch)')
     p.add_argument('--io-threads', type=int, default=8, help='loader and saver threads per GPU')
     p.add_argument('--raw-sink', default=None, metavar='PATH',
-                   help="hand the SBS frames to an encoder instead of writing sbs_*.png: raw rgb24, in clip order, into PATH "
+                   help="hand the SBS frames to an encoder instead of writing sbs_*.png: raw --pixfmt frames, in clip order, into PATH "
                         "(a file or FIFO; '-' = stdout); geometry in PATH.json.  Processes every frame pair (no resume)")
     p.add_argument('--layout', choices=LAYOUTS, default=None,
                    help="output frame layout (default: config.json \"sbs_layout\", else sbs): sbs [H,2W], half-sbs [H,W], "
                         "tb [2H,W], half-tb [H,W], anaglyph [H,W] (red-cyan)")
+    p.add_argument('--pixfmt', choices=PIXFMTS, default=None,
+                   help='pixel format of the frames (default: config.json "sbs_pixfmt", else rgb24); yuv420p and '
+                        'yuv420p10le (I420, limited range) need --raw-sink')
+    p.add_argument('--matrix', choices=MATRICES, default=None,
+                   help='YUV matrix of the yuv420 formats (default: config.json "sbs_matrix", else bt709)')
     return p
 
 
@@ -97,6 +104,19 @@ def layout_refusal(output_dir: Path, frame_path, layout: str):
     return None
 
 
+def format_refusal(frame_path, layout: str, pixfmt: str):
+    """Why `pixfmt` cannot take this clip's frames in `layout` (a YUV format needs whole 2x2 blocks), or None."""
+    from vsc_b200.stereo_core import output_shape
+    size = png_size(frame_path)
+    if size is None:
+        return None
+    try:
+        output_shape(layout, *size, pixfmt)
+    except ValueError as e:
+        return str(e)
+    return None
+
+
 def _decode_into(item, gen, slot, index, expected):
     """Loader job: decode one (frame, depth) pair.  When the pair has the clip's geometry and depth dtype the colour
     conversion writes straight into the slot's pinned input buffers (no staging copy); otherwise the arrays are
@@ -125,9 +145,10 @@ def _decode_into(item, gen, slot, index, expected):
         return 'error', str(e)
 
 
-def open_raw_sink(path: str, pairs, layout: str):
-    """RawFrameSink for `pairs` in clip order; frame geometry (and the JSON side-car) from the first frame and the
-    layout.  OSError when the first frame cannot be read, ValueError when the layout cannot take its size."""
+def open_raw_sink(path: str, pairs, layout: str, pixfmt: str = 'rgb24', matrix: str = 'bt709'):
+    """RawFrameSink for `pairs` in clip order; frame geometry (and the JSON side-car) from the first frame, the layout
+    and the pixel format.  OSError when the first frame cannot be read, ValueError when the layout or pixel format
+    cannot take its size."""
     import cv2
     from vsc_b200.sharder import RawFrameSink
     from vsc_b200.stereo_core import output_shape
@@ -135,12 +156,13 @@ def open_raw_sink(path: str, pairs, layout: str):
     if probe is None:
         raise OSError(f'cannot read {pairs[0][0]}')
     oh, ow, _ = output_shape(layout, probe.shape[0], probe.shape[1])
-    return RawFrameSink(path, len(pairs), oh, ow, frame_numbers=[p[2] for p in pairs])
+    output_shape(layout, probe.shape[0], probe.shape[1], pixfmt)       # refuses a size the pixel format cannot take
+    return RawFrameSink(path, len(pairs), oh, ow, frame_numbers=[p[2] for p in pairs], pixfmt=pixfmt, matrix=matrix)
 
 
 def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int, io_threads: int, free_space_mode: str,
                   no_interactive: bool, progress=None, sink=None, sink_index=None, group: int = 4, gen=None,
-                  layout: str = 'sbs') -> int:
+                  layout: str = 'sbs', pixfmt: str = 'rgb24', matrix: str = 'bt709') -> int:
     """Run `pairs` [(frame_path, depth_path, frame_num)] through one GPU.  Returns frames written.
 
     The pipeline the benchmark times: `slots` frame slots of `group` frames each.  A slot is filled by the loader
@@ -148,7 +170,8 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
     stream, one hole-filling launch for the group) and harvested with vsc_wait_any; finished frames go to the saver
     pool (bounded backlog) and become visible in frame order through the InOrderPublisher.
     With `sink` (a RawFrameSink shared by all GPUs of the process) frames go to it at position
-    `sink_index[frame_num]` instead of into sbs_<n>.png.  `layout` is the output layout of a generator made here."""
+    `sink_index[frame_num]` instead of into sbs_<n>.png.  `layout`, `pixfmt` and `matrix` set the output of a generator
+    made here (a YUV pixfmt only with a sink)."""
     import cv2
     import numpy as np
     from vsc_b200 import StereoGenerator
@@ -156,7 +179,8 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
 
     own_gen = gen is None         # a caller may pass a warm generator (n_slots >= slots, group_size >= group) and keep it
     if own_gen:
-        gen = StereoGenerator(f'cuda:{device_index}', n_slots=slots, group_size=group, layout=layout)
+        gen = StereoGenerator(f'cuda:{device_index}', n_slots=slots, group_size=group, layout=layout, pixfmt=pixfmt,
+                              matrix=matrix)
     loaders = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='load')
     savers = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='save')
     backlog = threading.BoundedSemaphore(max(2 * io_threads, group))     # frames waiting for / inside the savers
@@ -304,7 +328,7 @@ def main(argv=None) -> int:
         print(f'ERROR: Workflow directory not found: {args.workflow_path}')
         return 0
     ConfigError, get_path, load_config = _load_config_api()
-    from vsc_b200.workflow import LayoutError, config_layout
+    from vsc_b200.workflow import LayoutError, config_layout, config_pixfmt
     try:
         config = load_config(args.workflow_path)
     except ConfigError as e:
@@ -325,8 +349,13 @@ def main(argv=None) -> int:
         return 2
     try:
         layout = args.layout or config_layout(config)
+        cfg_pixfmt, cfg_matrix = config_pixfmt(config)
     except LayoutError as e:
         print(f'ERROR: {e}')
+        return 2
+    pixfmt, matrix = args.pixfmt or cfg_pixfmt, args.matrix or cfg_matrix
+    if pixfmt != 'rgb24' and not args.raw_sink:
+        print(f'ERROR: pixel format {pixfmt} is for the raw sink only (--raw-sink); sbs_*.png files are rgb24')
         return 2
 
     from vsc_b200 import StereoParams
@@ -350,7 +379,7 @@ def main(argv=None) -> int:
         if rank == 0:
             print('All frames already processed.')
         return 0
-    why = layout_refusal(output_dir, pairs[0][0], layout) if not args.raw_sink else None
+    why = layout_refusal(output_dir, pairs[0][0], layout) if not args.raw_sink else format_refusal(pairs[0][0], layout, pixfmt)
     if why:
         print(f'ERROR: {why}')
         return 2
@@ -365,7 +394,8 @@ def main(argv=None) -> int:
         print(f'Using GPU: {torch.cuda.get_device_name(0)} x{world if world > 1 else (args.gpus or ngpu)}')
         print(f'Parameters: disparity={params.max_disparity}, convergence={params.convergence}, '
               f'super_sampling={params.super_sampling}, edge_softness={params.edge_softness}, '
-              f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}, layout={layout}')
+              f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}, layout={layout}'
+              + (f', pixfmt={pixfmt}, matrix={matrix}' if pixfmt != 'rgb24' else ''))
 
     finals = [str(output_dir / f'sbs_{p[2]}.png') for p in pairs]
 
@@ -380,11 +410,11 @@ def main(argv=None) -> int:
             print('ERROR: --raw-sink needs all GPUs in one process (use --gpus N, not torchrun)')
             return 2
         try:
-            sink = open_raw_sink(args.raw_sink, pairs, layout)
+            sink = open_raw_sink(args.raw_sink, pairs, layout, pixfmt, matrix)
         except OSError as e:
             print(f'ERROR: {e}')
             return 0
-        except ValueError as e:         # the layout cannot take the frame size
+        except ValueError as e:         # the layout or pixel format cannot take the frame size
             print(f'ERROR: {e}')
             return 2
         sink_index = {p[2]: i for i, p in enumerate(pairs)}
@@ -425,7 +455,7 @@ def main(argv=None) -> int:
             t.start()
             if g == 1:
                 n = process_shard(pairs, output_dir, params, 0, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                                  sink, sink_index, args.group, layout=layout)
+                                  sink, sink_index, args.group, layout=layout, pixfmt=pixfmt, matrix=matrix)
             else:
                 # one worker thread per GPU; each owns a StereoGenerator (its own CUDA context state, streams, pinned ring)
                 results = [0] * g
@@ -435,7 +465,7 @@ def main(argv=None) -> int:
                     try:
                         results[k] = process_shard(shard_items(pairs, g, k), output_dir, params, k, args.slots, args.io_threads,
                                                    free_space_mode, args.no_interactive, progress, sink, sink_index, args.group,
-                                                   layout=layout)
+                                                   layout=layout, pixfmt=pixfmt, matrix=matrix)
                     except BaseException as e:   # noqa: BLE001
                         errors.append(e)
                 ths = [threading.Thread(target=work, args=(k,)) for k in range(g)]

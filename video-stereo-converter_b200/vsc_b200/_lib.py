@@ -16,6 +16,8 @@ LIB_PATH = os.environ.get('VSC_B200_LIB', os.path.normpath(os.path.join(_HERE, '
 VSC_OK, VSC_E_INVALID, VSC_E_PARAMS, VSC_E_CUDA, VSC_E_NOMEM, VSC_E_STATE = 0, -1, -2, -3, -4, -5
 DEPTH_U8, DEPTH_U16, DEPTH_F32 = 0, 1, 2
 LAYOUT_SBS, LAYOUT_HALF_SBS, LAYOUT_TB, LAYOUT_HALF_TB, LAYOUT_ANAGLYPH = 0, 1, 2, 3, 4
+PIXFMT_RGB24, PIXFMT_YUV420P, PIXFMT_YUV420P10LE = 0, 1, 2
+MATRIX_BT709, MATRIX_BT601 = 0, 1
 GPU_ERROR_EXIT_CODE = 100      # sbs_generator.py:41
 
 EXPORTS = [
@@ -27,7 +29,7 @@ EXPORTS = [
     'vsc_stage_backend', 'vsc_stage_depth_post', 'vsc_depth_post_device', 'vsc_stage_warp_f32', 'vsc_stage_normalize_f32', 'vsc_stage_gamma_f32',
     'vsc_set_profiling', 'vsc_slot_kernel_times', 'vsc_timer_begin', 'vsc_timer_end', 'vsc_debug_fetch',
     'vsc_debug_telea_state', 'vsc_debug_telea_stats', 'vsc_debug_set_telea_capacity', 'vsc_debug_selftest',
-    'vsc_layout_shape', 'vsc_set_layout',
+    'vsc_layout_shape', 'vsc_set_layout', 'vsc_output_size', 'vsc_set_pixfmt',
 ]
 
 
@@ -114,6 +116,8 @@ def load():
     lib.vsc_debug_selftest.argtypes = [vp, i, C.POINTER(C.c_ulonglong)]
     lib.vsc_layout_shape.argtypes = [i, i, i, C.POINTER(C.c_int), C.POINTER(C.c_int)]
     lib.vsc_set_layout.argtypes = [vp, i]
+    lib.vsc_output_size.argtypes = [i, i, i, i, C.POINTER(C.c_size_t)]
+    lib.vsc_set_pixfmt.argtypes = [vp, i, i]
     if lib.vsc_abi_version() != 1:
         raise ImportError('libvsc_b200.so ABI version mismatch')
     _lib = lib

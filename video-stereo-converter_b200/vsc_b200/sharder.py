@@ -161,11 +161,31 @@ class RawFrameSink:
     A JSON side-car (`<path>.json`, not written for '-') records the geometry and the frame numbers.
     `put` blocks while a frame is more than `max_ahead` positions ahead of the write cursor, so memory
     stays bounded when one GPU runs ahead of another.
+
+    `pixfmt` (stereo_core.PIXFMTS) is the format of the frames the library hands over: with 'yuv420p' or
+    'yuv420p10le' a frame is the I420 planes of a `width` x `height` picture as one [height * 3 // 2, width] array
+    (uint8 / uint16), limited range, centre-sited chroma, in `matrix`.  The encoder then reads its input format
+    directly, and the side-car's `ffmpeg_input` tags the stream's colour description, e.g.
+
+        ffmpeg -f rawvideo -pix_fmt yuv420p10le -s 3840x1080 -color_range tv -colorspace bt709 ... -i sbs.yuv ...
     """
 
-    def __init__(self, path: str, n_frames: int, height: int, width: int, max_ahead: int = 256, frame_numbers=None):
+    # ffmpeg's names of the colour description of each YUV matrix (-colorspace, -color_primaries, -color_trc)
+    _FFMPEG_COLOUR = {'bt709': 'bt709', 'bt601': 'smpte170m'}
+
+    def __init__(self, path: str, n_frames: int, height: int, width: int, max_ahead: int = 256, frame_numbers=None,
+                 pixfmt: str = 'rgb24', matrix: str = 'bt709'):
         import json
+        import numpy as np
+        from .stereo_core import matrix_code, output_dtype
         self.path, self.n, self.h, self.w = str(path), int(n_frames), int(height), int(width)
+        self.dtype = output_dtype(pixfmt)             # ValueError for an unknown format
+        matrix_code(matrix)
+        if pixfmt != 'rgb24' and (self.h % 2 or self.w % 2):
+            raise ValueError(f'{pixfmt} needs an even frame size, got {self.w}x{self.h}')
+        self.pixfmt, self.matrix = pixfmt, matrix
+        self.shape = (self.h, self.w, 3) if pixfmt == 'rgb24' else (self.h * 3 // 2, self.w)
+        self.bytes_per_frame = int(np.prod(self.shape)) * self.dtype.itemsize
         self.max_ahead = int(max_ahead)
         self._pending = {}
         self._next = 0
@@ -177,17 +197,23 @@ class RawFrameSink:
             self._f = sys.__stdout__.buffer     # the driver moves its own messages to stderr in this mode
         else:
             self._f = open(self.path, 'wb')
+            meta = {'pix_fmt': pixfmt, 'width': self.w, 'height': self.h, 'frames': self.n,
+                    'bytes_per_frame': self.bytes_per_frame,
+                    'frame_numbers': list(frame_numbers) if frame_numbers is not None else None,
+                    'ffmpeg_input': f'-f rawvideo -pix_fmt rgb24 -s {self.w}x{self.h} -i {self.path}'}
+            if pixfmt != 'rgb24':
+                c = self._FFMPEG_COLOUR[matrix]
+                meta.update(matrix=matrix, range='tv', chroma_location='center',
+                            ffmpeg_input=f'-f rawvideo -pix_fmt {pixfmt} -s {self.w}x{self.h} -color_range tv -colorspace {c} '
+                                         f'-color_primaries {c} -color_trc {c} -i {self.path}')
             with open(self.path + '.json', 'w') as jf:
-                json.dump({'pix_fmt': 'rgb24', 'width': self.w, 'height': self.h, 'frames': self.n,
-                           'bytes_per_frame': self.w * self.h * 3,
-                           'frame_numbers': list(frame_numbers) if frame_numbers is not None else None,
-                           'ffmpeg_input': f'-f rawvideo -pix_fmt rgb24 -s {self.w}x{self.h} -i {self.path}'}, jf)
+                json.dump(meta, jf)
         self._t = threading.Thread(target=self._run, name='raw-sink', daemon=True)
         self._t.start()
 
     def put(self, index: int, frame) -> None:
-        if frame.shape != (self.h, self.w, 3) or str(frame.dtype) != 'uint8':
-            raise ValueError(f'frame {index}: expected uint8 {(self.h, self.w, 3)}, got {frame.dtype} {frame.shape}')
+        if frame.shape != self.shape or frame.dtype != self.dtype:
+            raise ValueError(f'frame {index}: expected {self.dtype} {self.shape}, got {frame.dtype} {frame.shape}')
         with self._cv:
             while index - self._next > self.max_ahead and self._error is None:
                 self._cv.wait(0.1)
@@ -197,9 +223,16 @@ class RawFrameSink:
             self._cv.notify_all()
 
     def skip(self, index: int) -> None:
-        """A frame that could not be produced (load error): keep the stream gap-free with a black frame."""
+        """A frame that could not be produced (load error): keep the stream gap-free with a black frame (in YUV:
+        Y 16 / 64, chroma 128 / 512 at 8 / 10 bits)."""
         import numpy as np
-        self.put(index, np.zeros((self.h, self.w, 3), np.uint8))
+        if self.pixfmt == 'rgb24':
+            self.put(index, np.zeros(self.shape, np.uint8))
+            return
+        black = np.empty(self.shape, self.dtype)
+        black[:self.h] = 16 if self.pixfmt == 'yuv420p' else 64
+        black[self.h:] = 128 if self.pixfmt == 'yuv420p' else 512
+        self.put(index, black)
 
     @property
     def written(self) -> int:

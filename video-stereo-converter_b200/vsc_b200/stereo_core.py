@@ -8,7 +8,9 @@ sm_100a CUDA kernels behind the C ABI of include/vsc_b200.h.  There is no CPU pa
 Additions that the reference does not have (used by the frame loop in sbs_generator.py):
 `StereoGenerator.submit/collect` (asynchronous, pinned, multi-slot) and `process_batch`, and output layouts
 (`StereoGenerator(..., layout='half-sbs')`, `LAYOUTS`, `output_shape`): every output path then returns frames of
-`output_shape(layout, h, w)` instead of the side-by-side [h, 2w, 3].
+`output_shape(layout, h, w)` instead of the side-by-side [h, 2w, 3].  Output pixel formats
+(`StereoGenerator(..., pixfmt='yuv420p10le', matrix='bt709')`, `PIXFMTS`, `MATRICES`, `output_dtype`): the YUV formats
+return the I420 planes of that frame as one [rows * 3 // 2, cols] array, the shape cv2's COLOR_RGB2YUV_I420 uses.
 """
 from __future__ import annotations
 
@@ -55,15 +57,48 @@ def layout_code(layout: str) -> int:
     return LAYOUTS.index(layout)
 
 
-def output_shape(layout: str, h: int, w: int) -> Tuple[int, int, int]:
-    """Shape (rows, cols, 3) of the frame `layout` makes of an h x w input (the library's vsc_layout_shape).
-    ValueError for an unknown layout or an odd side that a half layout halves."""
+# output pixel formats (include/vsc_b200.h VSC_PIXFMT_*) and the matrices of the YUV formats (VSC_MATRIX_*):
+# name -> C enum, named as ffmpeg names them.  'rgb24' is the reference's output.
+PIXFMTS = ('rgb24', 'yuv420p', 'yuv420p10le')
+MATRICES = ('bt709', 'bt601')
+
+
+def pixfmt_code(pixfmt: str) -> int:
+    """C enum of a pixel format name; ValueError for anything else."""
+    if pixfmt not in PIXFMTS:
+        raise ValueError(f'unknown pixel format {pixfmt!r} (one of {", ".join(PIXFMTS)})')
+    return PIXFMTS.index(pixfmt)
+
+
+def matrix_code(matrix: str) -> int:
+    """C enum of a YUV matrix name; ValueError for anything else."""
+    if matrix not in MATRICES:
+        raise ValueError(f'unknown yuv matrix {matrix!r} (one of {", ".join(MATRICES)})')
+    return MATRICES.index(matrix)
+
+
+def output_dtype(pixfmt: str) -> np.dtype:
+    """Element type of the frames of a pixel format: uint16 (value in the low 10 bits) for yuv420p10le, else uint8."""
+    return np.dtype(np.uint16 if pixfmt_code(pixfmt) == _lib.PIXFMT_YUV420P10LE else np.uint8)
+
+
+def output_shape(layout: str, h: int, w: int, pixfmt: str = 'rgb24') -> Tuple[int, ...]:
+    """Shape (rows, cols, 3) of the frame `layout` makes of an h x w input (the library's vsc_layout_shape).  For a YUV
+    pixel format: (rows * 3 // 2, cols), the I420 planes Y [rows][cols], U and V [rows/2][cols/2] one after the other.
+    ValueError for an unknown layout or format, or a size they cannot take (an odd side that a half layout halves; for
+    YUV an odd side, or a width (half-sbs) or height (half-tb) not divisible by 4)."""
     code = layout_code(layout)
     oh, ow = C.c_int(), C.c_int()
     rc = _lib.load().vsc_layout_shape(code, int(h), int(w), C.byref(oh), C.byref(ow))
     if rc != _lib.VSC_OK:
         raise ValueError((_lib.load().vsc_last_error() or b'').decode('utf-8', 'replace'))
-    return oh.value, ow.value, 3
+    if pixfmt_code(pixfmt) == _lib.PIXFMT_RGB24:
+        return oh.value, ow.value, 3
+    n = C.c_size_t()
+    rc = _lib.load().vsc_output_size(code, pixfmt_code(pixfmt), int(h), int(w), C.byref(n))
+    if rc != _lib.VSC_OK:
+        raise ValueError((_lib.load().vsc_last_error() or b'').decode('utf-8', 'replace'))
+    return oh.value * 3 // 2, ow.value
 
 
 # ------------------------------------------------------------------------------------------------
@@ -182,17 +217,20 @@ class StereoGenerator:
 
     `process_frame(rgb, depth, params)` keeps the reference's numpy-in / numpy-out contract.
     `n_slots` frames can be in flight through `submit` / `collect` for the driver loop.
-    `layout` (one of LAYOUTS, default the reference's 'sbs') sets the shape of every frame this generator returns.
+    `layout` (one of LAYOUTS, default the reference's 'sbs') sets the shape of every frame this generator returns, and
+    `pixfmt` (one of PIXFMTS, default 'rgb24') with `matrix` (one of MATRICES, for the YUV formats) its pixel format.
     """
     _DEFAULT_PARAMS = StereoParams()
 
-    def __init__(self, device: str, n_slots: int = 1, group_size: int = 1, layout: str = 'sbs') -> None:
+    def __init__(self, device: str, n_slots: int = 1, group_size: int = 1, layout: str = 'sbs', pixfmt: str = 'rgb24',
+                 matrix: str = 'bt709') -> None:
         self.device = device
-        code = layout_code(layout)
+        code, fcode, mcode = layout_code(layout), pixfmt_code(pixfmt), matrix_code(matrix)
         self._ctx = _lib.Context(_parse_device(device), n_slots, group_size)
         self._lib = _lib.load()
         _lib.check(self._lib.vsc_set_layout(self._ctx.handle, code))
-        self.layout = layout
+        _lib.check(self._lib.vsc_set_pixfmt(self._ctx.handle, fcode, mcode))
+        self.layout, self.pixfmt, self.matrix = layout, pixfmt, matrix
         self.n_slots, self.group_size = n_slots, group_size
         self._pending = [None] * n_slots        # per slot: number of frames in flight
         # pinned staging per (slot, frame index within the slot's group): (key, rgb, depth, out) PinnedBuffers
@@ -201,11 +239,11 @@ class StereoGenerator:
     # -- reference API ---------------------------------------------------------------------------
     def process_frame(self, rgb: np.ndarray, depth: np.ndarray, params: StereoParams | None = None) -> np.ndarray:
         """Process a single frame to a side-by-side stereo image (left | right), uint8 [H, 2W, 3]
-        (with another layout: uint8 of output_shape(layout, H, W))."""
+        (with another layout or pixel format: output_shape(layout, H, W, pixfmt) of output_dtype(pixfmt))."""
         p = params or self._DEFAULT_PARAMS
         rgb_c, depth_c, code = self._check_inputs(rgb, depth)
         h, w = rgb_c.shape[:2]
-        out = np.empty(self.output_shape(h, w), np.uint8)
+        out = np.empty(self.output_shape(h, w), self.output_dtype)
         _lib.check(self._lib.vsc_process_frame(self._ctx.handle, _lib.ptr(rgb_c), _lib.ptr(depth_c), code, h, w,
                                                C.byref(_lib.make_params(p)), _lib.ptr(out)))
         return out
@@ -214,7 +252,7 @@ class StereoGenerator:
     def pinned_inputs(self, slot: int, h: int, w: int, depth_dtype=np.uint8, index: int = 0):
         """Page-locked (rgb[h,w,3], depth[h,w]) arrays of frame `index` of `slot` for a loader to decode into."""
         key = (int(h), int(w), np.dtype(depth_dtype).str)
-        self.output_shape(h, w)             # a size the layout cannot take is refused before any buffer changes
+        self.output_shape(h, w)             # a size the layout or format cannot take is refused before any buffer changes
         pin = self._pinned[slot][index]
         if pin is None or pin[0] != key:
             if self._pending[slot] is not None:
@@ -223,7 +261,7 @@ class StereoGenerator:
                 for b in pin[1:]:
                     b.free()
             pin = (key, _lib.PinnedBuffer((h, w, 3), np.uint8), _lib.PinnedBuffer((h, w), depth_dtype),
-                   _lib.PinnedBuffer(self.output_shape(h, w), np.uint8))
+                   _lib.PinnedBuffer(self.output_shape(h, w), self.output_dtype))
             self._pinned[slot][index] = pin
         return pin[1].array, pin[2].array
 
@@ -312,7 +350,7 @@ class StereoGenerator:
     def submit_device(self, slot: int, d_rgb: int, d_depth: int, depth_dtype, h: int, w: int, d_out: int,
                       params: StereoParams | None = None) -> None:
         """Device-resident variant: raw device pointers (e.g. torch tensor .data_ptr()), no copies.  d_out must hold
-        output_shape(h, w) uint8."""
+        output_shape(h, w) of output_dtype (self.output_shape, self.output_dtype)."""
         p = params or self._DEFAULT_PARAMS
         _lib.check(self._lib.vsc_submit_device(self._ctx.handle, slot, C.c_void_p(d_rgb), C.c_void_p(d_depth),
                                                _lib.depth_code(depth_dtype), h, w, C.byref(_lib.make_params(p)),
@@ -449,17 +487,36 @@ class StereoGenerator:
             raise RuntimeError('collect every slot before changing the layout')
         _lib.check(self._lib.vsc_set_layout(self._ctx.handle, code))
         self.layout = layout
+        self._release_pinned()
+
+    def set_pixfmt(self, pixfmt: str, matrix: str = 'bt709') -> None:
+        """Switch the pixel format (and YUV matrix) of frames submitted from now on.  Every slot must be collected, as for
+        set_layout."""
+        fcode, mcode = pixfmt_code(pixfmt), matrix_code(matrix)
+        if any(x is not None for x in self._pending):
+            raise RuntimeError('collect every slot before changing the pixel format')
+        _lib.check(self._lib.vsc_set_pixfmt(self._ctx.handle, fcode, mcode))
+        self.pixfmt, self.matrix = pixfmt, matrix
+        self._release_pinned()
+
+    # -- helpers -----------------------------------------------------------------------------------
+    def output_shape(self, h: int, w: int) -> Tuple[int, ...]:
+        """Shape of the frames this generator returns for h x w inputs."""
+        return output_shape(self.layout, h, w, self.pixfmt)
+
+    @property
+    def output_dtype(self) -> np.dtype:
+        """Element type of the frames this generator returns."""
+        return output_dtype(self.pixfmt)
+
+    def _release_pinned(self) -> None:
+        """Free the pinned buffers of every slot (pinned_inputs allocates them again in the current output shape)."""
         for row in self._pinned:
             for i, pin in enumerate(row):
                 if pin is not None:
                     for b in pin[1:]:
                         b.free()
                     row[i] = None
-
-    # -- helpers -----------------------------------------------------------------------------------
-    def output_shape(self, h: int, w: int) -> Tuple[int, int, int]:
-        """Shape of the frames this generator returns for h x w inputs."""
-        return output_shape(self.layout, h, w)
 
     @staticmethod
     def _check_inputs(rgb: np.ndarray, depth: np.ndarray):

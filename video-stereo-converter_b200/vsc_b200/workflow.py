@@ -7,7 +7,9 @@ keys this stage needs, so that sbs_generator.py runs both inside the reference t
 
 One key is this implementation's own: the optional top-level "sbs_layout" (output layout of the SBS stage, one of
 stereo_core.LAYOUTS, default "sbs").  It sits at the top level because the reference's validator accepts extra
-top-level keys while the reference builds StereoParams from the whole `stereo` block.
+top-level keys while the reference builds StereoParams from the whole `stereo` block.  So do the optional
+"sbs_pixfmt" (pixel format of the frames, one of stereo_core.PIXFMTS, default "rgb24") and "sbs_matrix" (YUV matrix, one
+of stereo_core.MATRICES, default "bt709").
 """
 from __future__ import annotations
 
@@ -18,6 +20,7 @@ from typing import Dict
 STEREO_KEYS = ('max_disparity', 'convergence', 'super_sampling', 'edge_softness', 'artifact_smoothing', 'depth_gamma', 'sharpen')
 DIR_KEYS = ('frames', 'depth_maps', 'sbs')
 LAYOUT_KEY = 'sbs_layout'
+PIXFMT_KEY, MATRIX_KEY = 'sbs_pixfmt', 'sbs_matrix'
 
 
 class ConfigError(Exception):
@@ -25,7 +28,8 @@ class ConfigError(Exception):
 
 
 class LayoutError(ConfigError):
-    """The optional "sbs_layout" key holds something other than a layout name."""
+    """One of the optional output keys ("sbs_layout", "sbs_pixfmt", "sbs_matrix") holds something other than a name
+    it takes."""
 
 
 def config_layout(cfg: Dict) -> str:
@@ -35,6 +39,18 @@ def config_layout(cfg: Dict) -> str:
     if v not in LAYOUTS:
         raise LayoutError(f"Invalid '{LAYOUT_KEY}' {v!r} (expected one of {', '.join(LAYOUTS)})")
     return v
+
+
+def config_pixfmt(cfg: Dict):
+    """(pixel format, yuv matrix) a config asks for: top-level "sbs_pixfmt" and "sbs_matrix", default ('rgb24', 'bt709')."""
+    from .stereo_core import MATRICES, PIXFMTS
+    out = []
+    for key, names, default in ((PIXFMT_KEY, PIXFMTS, 'rgb24'), (MATRIX_KEY, MATRICES, 'bt709')):
+        v = cfg.get(key, default)
+        if v not in names:
+            raise LayoutError(f"Invalid '{key}' {v!r} (expected one of {', '.join(names)})")
+        out.append(v)
+    return tuple(out)
 
 
 def load_config(workflow_path) -> Dict:
@@ -58,6 +74,7 @@ def load_config(workflow_path) -> Dict:
         if isinstance(v, bool) or not isinstance(v, (int, float)):
             raise ConfigError(f"Missing or invalid 'stereo.{k}' (expected float)")
     config_layout(cfg)
+    config_pixfmt(cfg)
     return cfg
 
 
