@@ -10,6 +10,8 @@ cv2 = pytest.importorskip('cv2')
 torch = pytest.importorskip('torch')
 F = torch.nn.functional
 
+from helper_reference import warp_literal  # noqa: E402  (needs torch)
+
 
 @pytest.mark.parametrize('h,w,dw', [(37, 160, 270), (12, 1920, 2030), (6, 3840, 3949), (11, 100, 137)])
 def test_lanczos4_bit_exact_vs_cv2(h, w, dw):
@@ -106,34 +108,6 @@ def test_pow_specification_tables_and_accuracy():
     assert np.array_equal(O.apply_gamma(x, 2.0), x * x) and np.array_equal(O.apply_gamma(x, 3.0), (x * x) * x)
 
 
-def _warp_literal_torch(image, depth, md, sign):
-    """forward_warp_stereo's algorithm, stated literally: ascending-depth argsort, floor scatters, then
-    ceil scatters of the frac > 0.3 subset, last writer wins."""
-    c, h, w = image.shape
-    d = torch.from_numpy(depth).flatten()
-    order = torch.argsort(d)
-    ys = (torch.arange(h * w) // w)[order]
-    xs = (torch.arange(h * w) % w).float()[order]
-    tx = xs + sign * (d * md)[order]
-    fl = tx.floor().long()
-    frac = tx - fl.float()
-    img = torch.from_numpy(image).reshape(c, -1)
-    out = torch.zeros(c, h * w)
-    wgt = torch.zeros(h * w)
-    ok = (fl >= 0) & (fl < w)
-    idx = (ys * w + fl)[ok]
-    for ch in range(c):
-        out[ch].scatter_(0, idx, img[ch, order[ok]])
-    wgt.scatter_(0, idx, (1.0 - frac)[ok])
-    ce = fl + 1
-    ok = (ce >= 0) & (ce < w) & (frac > 0.3)
-    idx = (ys * w + ce)[ok]
-    for ch in range(c):
-        out[ch].scatter_(0, idx, img[ch, order[ok]])
-    wgt.scatter_(0, idx, frac[ok])
-    return out.reshape(c, h, w).numpy(), (wgt > 0.1).reshape(h, w).numpy().astype(np.uint8)
-
-
 @pytest.mark.parametrize('kind', ['random', 'ties', 'ramp'])
 def test_sort_free_warp_equals_literal_argsort_scatter(kind):
     rng = np.random.default_rng(5)
@@ -146,7 +120,7 @@ def test_sort_free_warp_equals_literal_argsort_scatter(kind):
     else:
         dep = np.tile(np.linspace(0, 1, w, dtype=np.float32)[None] ** 3, (h, 1))
     for sign in (+1, -1):
-        ref_img, ref_mask = _warp_literal_torch(img, dep, md, sign)
+        ref_img, ref_mask = warp_literal(img, dep, md, sign)
         mine_img, mine_mask = O.warp(img, dep, md, sign)
         assert np.array_equal(mine_mask, ref_mask) and np.array_equal(mine_img, ref_img)
 

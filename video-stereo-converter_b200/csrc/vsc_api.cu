@@ -1303,12 +1303,14 @@ extern "C" int vsc_stage_warp_f32(vsc_ctx* ctx, const float* image, const float*
     CU(cudaMemcpyAsync(dd.p, depth, n * 4, cudaMemcpyHostToDevice, s.stream));
     CU(cudaMemsetAsync(o0.p, 0, n * C * 4, s.stream)); CU(cudaMemsetAsync(o1.p, 0, n * C * 4, s.stream));
     CU(cudaMemsetAsync(m0.p, 0, n * 4, s.stream)); CU(cudaMemsetAsync(m1.p, 0, n * 4, s.stream));
+    // the depth's extremes bound how far a source moves, i.e. the halo each segment scans (the depth may be unnormalised)
+    minmax_kernel<<<ctx->sm_count * 4, kThreads, 0, s.stream>>>((const float*)dd.p, n, s.scalars.as<FrameScalars>());
     const int nseg = (W + 1023) / 1024;
     const int TS = (int)align_up((size_t)(W + nseg - 1) / nseg, 32);
-    const int R = (int)ceil(fabs(md)) + 1;
     dim3 grid(nseg, H);
-    warp_f32_kernel<<<grid, kThreads, (size_t)TS * 16, s.stream>>>((const float*)di.p, (const float*)dd.p, C, H, W, (float)md, R, TS,
-                                                                  (float*)o0.p, (float*)m0.p, (float*)o1.p, (float*)m1.p);
+    warp_f32_kernel<<<grid, kThreads, (size_t)TS * 16, s.stream>>>((const float*)di.p, (const float*)dd.p, C, H, W, (float)md,
+                                                                  s.scalars.as<FrameScalars>(), TS, (float*)o0.p, (float*)m0.p,
+                                                                  (float*)o1.p, (float*)m1.p);
     KCHECK(s);
     CU(cudaMemcpyAsync(left, o0.p, n * C * 4, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaMemcpyAsync(right, o1.p, n * C * 4, cudaMemcpyDeviceToHost, s.stream));

@@ -15,6 +15,7 @@ return the I420 planes of that frame as one [rows * 3 // 2, cols] array, the sha
 from __future__ import annotations
 
 import ctypes as C
+import threading
 from dataclasses import dataclass
 from pathlib import Path
 from typing import Iterable, List, Optional, Tuple
@@ -130,9 +131,13 @@ def _resize_depth_to(depth: np.ndarray, w: int, h: int) -> np.ndarray:
 # shared default context for the module-level helpers
 # ------------------------------------------------------------------------------------------------
 _default_ctx: Optional[_lib.Context] = None
+# The helpers share _default_ctx, i.e. one stream and one set of device scalars (its slot 0), and ctypes releases the
+# GIL during a call: every use of that context holds this lock, so concurrent helper calls run one after the other.
+_helper_lock = threading.Lock()
 
 
 def _ctx() -> _lib.Context:
+    """The helpers' shared context; call with _helper_lock held."""
     global _default_ctx
     if _default_ctx is None:
         _default_ctx = _lib.Context(_current_device(), 1)
@@ -150,7 +155,8 @@ def _current_device() -> int:
 
 
 def _as_f32(t):
-    """torch tensor -> contiguous float32 numpy on host (+ a function to map results back)."""
+    """torch tensor -> contiguous float32 numpy on host (+ a function to map results back).  The helpers compute in
+    float32 whatever the input's dtype, and cast the results back to it."""
     import torch
     if not isinstance(t, torch.Tensor):
         raise TypeError('expected a torch.Tensor')
@@ -166,7 +172,8 @@ def normalize_depth(depth):
     """Normalize depth to [0, 1] (reference: stereo_core.py:71-88); zeros if the range is < 1e-6."""
     a, back = _as_f32(depth)
     out = np.empty_like(a)
-    _lib.check(_lib.load().vsc_stage_normalize_f32(_ctx().handle, _lib.ptr(a), a.size, _lib.ptr(out)))
+    with _helper_lock:
+        _lib.check(_lib.load().vsc_stage_normalize_f32(_ctx().handle, _lib.ptr(a), a.size, _lib.ptr(out)))
     return back(out)
 
 
@@ -174,7 +181,8 @@ def apply_depth_gamma(depth, gamma: float):
     """pow(clamp(depth, 0.001, 1), gamma) (reference: stereo_core.py:91-107)."""
     a, back = _as_f32(depth)
     out = np.empty_like(a)
-    _lib.check(_lib.load().vsc_stage_gamma_f32(_ctx().handle, _lib.ptr(a), a.size, float(gamma), _lib.ptr(out)))
+    with _helper_lock:
+        _lib.check(_lib.load().vsc_stage_gamma_f32(_ctx().handle, _lib.ptr(a), a.size, float(gamma), _lib.ptr(out)))
     return back(out)
 
 
@@ -193,8 +201,9 @@ def forward_warp_stereo(image, depth, max_disparity: float):
         raise RuntimeError('depth must have H*W elements')
     left, right = np.empty((1, c, h, w), np.float32), np.empty((1, c, h, w), np.float32)
     lm, rm = np.empty((1, 1, h, w), np.float32), np.empty((1, 1, h, w), np.float32)
-    _lib.check(_lib.load().vsc_stage_warp_f32(_ctx().handle, _lib.ptr(img), _lib.ptr(dep), c, h, w, float(max_disparity),
-                                              _lib.ptr(left), _lib.ptr(lm), _lib.ptr(right), _lib.ptr(rm)))
+    with _helper_lock:
+        _lib.check(_lib.load().vsc_stage_warp_f32(_ctx().handle, _lib.ptr(img), _lib.ptr(dep), c, h, w, float(max_disparity),
+                                                  _lib.ptr(left), _lib.ptr(lm), _lib.ptr(right), _lib.ptr(rm)))
     return back(left), back(lm), back(right), back(rm)
 
 
