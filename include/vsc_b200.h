@@ -163,6 +163,34 @@ int vsc_output_size(int layout, int pixfmt, int height, int width, size_t *bytes
  * launch is added: the conversion is the store epilogue of the back-end kernel.  vsc_stage_backend always writes RGB24. */
 int vsc_set_pixfmt(vsc_ctx *ctx, int pixfmt, int matrix);
 
+/* -------- encoded output (no reference counterpart) -------------------------------------------- */
+/* VSC_ENCODE_PNG: every frame leaves the library as a complete PNG file of its rgb24 frame in the chosen layout
+ * (oh x ow, 8-bit truecolour, chunks IHDR, IDAT..., IEND), encoded on the device by three kernels after the back end:
+ *   filter   per row the PNG filter 0..4 of least sum(min(b, 256 - b)) over its filtered bytes (ties: the lowest type;
+ *            row 0 against a zero row): the filtered stream, N = oh * (1 + 3 ow) bytes
+ *   zlib     78 01, then per 32768-byte segment of the filtered stream (segments ignore row edges) one deflate block of
+ *            its own: a greedy run-length parse (literals and distance-1 matches of 3..258, zlib's Z_RLE, no match
+ *            reaching before the segment), dynamic Huffman (lit/len codes <= 15 bits, code-length codes <= 7 bits, one
+ *            1-bit distance code), or stored when that is not larger; each segment is followed by an empty stored block
+ *            (sync flush), so segments are byte-aligned.  Then a final empty fixed block (03 00) and the Adler-32.
+ *   framing  one IDAT per segment; the first also holds the zlib header, the last the final block and the Adler-32.
+ * Worst case (the capacity an output buffer must have), with nseg = ceil(N / 32768):
+ *   bytes = 53 + N + 22 * nseg
+ * PNG needs VSC_PIXFMT_RGB24: vsc_set_encode refuses PNG under a YUV format, vsc_set_pixfmt refuses a YUV format under
+ * PNG, and a submission with both fails, all with VSC_E_INVALID. */
+enum { VSC_ENCODE_NONE = 0, VSC_ENCODE_PNG = 1 };
+/* encoding of frames submitted to ctx from now on (like vsc_set_layout: frames in flight keep theirs).  Default NONE.
+ * With PNG every submit path (vsc_process_frame, vsc_submit*, vsc_submit_device*) writes the file into the out buffer,
+ * which must hold vsc_encoded_capacity bytes.  A page-locked host buffer (vsc_host_alloc) is written by the device
+ * directly, so that only the file's bytes cross the bus; a pageable one receives the whole capacity after the run. */
+int vsc_set_encode(vsc_ctx *ctx, int encode);
+/* host only: the worst-case file bytes of an H x W input in (layout, encode) (NONE: the rgb24 frame's bytes);
+ * VSC_E_INVALID for an unknown layout or encoding or a size the layout cannot take */
+int vsc_encoded_capacity(int layout, int encode, int height, int width, size_t *bytes);
+/* bytes of the file of frame `index` of the slot's last completed submission (VSC_E_STATE while it is in flight or
+ * if that submission was not encoded) */
+int vsc_encoded_bytes(vsc_ctx *ctx, int slot, int index, size_t *bytes);
+
 /* -------- stage-level entry points for per-stage parity tests (host buffers, synchronous) --- */
 /* cv2.resize(src,(dst_w,H),INTER_LANCZOS4) (stereo_core.py:253-254); channels 1 or 3 for u8 */
 int vsc_stage_lanczos(vsc_ctx *ctx, const void *src, int dtype, int channels, int height, int width,
@@ -191,6 +219,11 @@ int vsc_stage_inpaint(vsc_ctx *ctx, uint8_t *img, const uint8_t *valid, int heig
 int vsc_stage_backend(vsc_ctx *ctx, const uint8_t *left, const uint8_t *right, int ss_h, int ss_w,
                       int left_crop, int right_crop, int crop_w, int height, int width, double sharpen,
                       uint8_t *out_sbs);
+
+/* The PNG encoding of VSC_ENCODE_PNG applied to an arbitrary rgb24 frame rgb [H][W][3] (host buffers, synchronous):
+ * the file goes to out (capacity >= vsc_encoded_capacity(VSC_LAYOUT_ANAGLYPH, VSC_ENCODE_PNG, H, W), the layout that
+ * keeps H x W), its size to *bytes. */
+int vsc_stage_png(vsc_ctx *ctx, const uint8_t *rgb, int height, int width, uint8_t *out, size_t capacity, size_t *bytes);
 
 /* Depth-map post-processing of the producer stage (/root/reference/depth_map_generator.py:217-236, SURVEY.md 8(f) rank 3):
  * cv2.resize(depth f32 [h,w] -> [H,W], INTER_LINEAR), min/max normalise, x255 (bits 8) or x65535 (bits 16), round half to
@@ -234,6 +267,9 @@ int vsc_debug_set_telea_capacity(vsc_ctx *ctx, size_t entries);
  * their range: which = 0 reciprocal (MUFU.RCP + one Newton step) against the correctly rounded 1/x on [1, 256);
  * which = 1 x/3 by multiply + two FMAs against the IEEE quotient on [0, 2295].  *mismatches must come back 0. */
 int vsc_debug_selftest(vsc_ctx *ctx, int which, unsigned long long *mismatches);
+/* counters of the last vsc_stage_png call: out[0] segments whose lit/len code needed the 15-bit limit, out[1] segments
+ * whose code-length code needed the 7-bit limit, out[2] segments written as stored blocks */
+int vsc_debug_png_stats(vsc_ctx *ctx, unsigned long long *out);
 
 #ifdef __cplusplus
 }

@@ -22,6 +22,7 @@
 
 #include "../../include/vsc_b200.h"
 #include "vsc_march.cuh"
+#include "vsc_png.cuh"
 
 using namespace vsc;
 
@@ -250,7 +251,11 @@ struct Slot {
     DevBuf scalars;     // FrameScalars
     DevBuf tstats;      // Telea phase counters (VSC_TELEA_STATS builds)
     DevBuf dp_scalars;  // min / max of the depth post-processing stage
+    DevBuf png_work;    // PNG: filtered stream, segment blocks, segment metadata, file size
+    DevBuf png_stage;   // PNG file of a submission whose host destination is pageable
+    DevBuf png_stats;   // PNG debug counters (vsc_stage_png)
     FrameScalars* h_scalars = nullptr;   // pinned mirror
+    unsigned long long* h_png = nullptr; // pinned: bytes of the PNG file of the last submission
     // table cache key
     int kH = 0, kW = 0, kSW = 0, kHs = 0, kWs = 0;
     const int* d_sx0 = nullptr; const short* d_it = nullptr; const float* d_ft = nullptr;
@@ -263,6 +268,9 @@ struct Slot {
     int l_dtype = 0, l_H = 0, l_W = 0; vsc_params l_p; uint8_t* l_host_out = nullptr; size_t l_out_bytes = 0;
     int l_layout = VSC_LAYOUT_SBS;       // output layout of the frame in this slot (fixed at submission)
     int l_pixfmt = VSC_PIXFMT_RGB24, l_matrix = VSC_MATRIX_BT709;   // its pixel format and YUV matrix (the same)
+    int l_encode = VSC_ENCODE_NONE;      // its encoding (the same); with PNG, l_out holds the rgb24 frame and l_png the file
+    uint8_t* l_png = nullptr;            // device-accessible destination of the PNG file
+    const uint8_t* l_copy_src = nullptr; // device source of the copy into l_host_out (l_out_bytes bytes)
     int launches = 0;
     float last_ms = 0.f;
     bool done = false;                   // leader only: the stream has run past the submission (set by a host callback)
@@ -281,6 +289,7 @@ struct vsc_ctx {
     int layout = VSC_LAYOUT_SBS;         // output layout of frames submitted from now on (vsc_set_layout)
     int pixfmt = VSC_PIXFMT_RGB24;       // pixel format and YUV matrix of frames submitted from now on (vsc_set_pixfmt)
     int matrix = VSC_MATRIX_BT709;
+    int encode = VSC_ENCODE_NONE;        // encoding of frames submitted from now on (vsc_set_encode)
     cudaStream_t tstream = nullptr;
     cudaEvent_t t0 = nullptr, t1 = nullptr;
     std::vector<cudaEvent_t> tslot;
@@ -378,6 +387,7 @@ static int set_smem_attrs() {
     if ((rc = backend_attrs<0>(big)) || (rc = backend_attrs<2>(big)) || (rc = backend_attrs<3>(big)) || (rc = backend_attrs<4>(big))) return rc;
     CU(cudaFuncSetAttribute(telea_march_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MarchSh<16>)));
     CU(cudaFuncSetAttribute(telea_march_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MarchSh<32>)));
+    CU(cudaFuncSetAttribute(png_segment_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PNG_SEG_SMEM));
     return VSC_OK;
 }
 
@@ -413,12 +423,14 @@ extern "C" int vsc_create_grouped(int device, int n_groups, int group_size, vsc_
             s.stream = ctx->slots[i - i % group_size].stream;
         }
         ok = ok && cudaEventCreate(&s.ev0) == cudaSuccess && cudaEventCreate(&s.ev1) == cudaSuccess &&
-             cudaMallocHost((void**)&s.h_scalars, sizeof(FrameScalars)) == cudaSuccess;
+             cudaMallocHost((void**)&s.h_scalars, sizeof(FrameScalars)) == cudaSuccess &&
+             cudaMallocHost((void**)&s.h_png, sizeof(unsigned long long)) == cudaSuccess;
         if (!ok) {
             vsc_destroy(ctx);
             return fail(VSC_E_CUDA, "failed to create stream/events for a slot");
         }
         memset(s.h_scalars, 0, sizeof(FrameScalars));
+        *s.h_png = 0;
     }
     *out = ctx;
     return VSC_OK;
@@ -438,8 +450,12 @@ extern "C" void vsc_destroy(vsc_ctx* ctx) {
         for (DevBuf* b : bufs) b->release();
         s.tstats.release();
         s.dp_scalars.release();
+        s.png_work.release();
+        s.png_stage.release();
+        s.png_stats.release();
         for (cudaEvent_t e : s.pev) cudaEventDestroy(e);
         if (s.h_scalars) cudaFreeHost(s.h_scalars);
+        if (s.h_png) cudaFreeHost(s.h_png);
         if (s.ev0) cudaEventDestroy(s.ev0);
         if (s.ev1) cudaEventDestroy(s.ev1);
         if (s.stream && s.owns_stream) cudaStreamDestroy(s.stream);
@@ -768,6 +784,41 @@ static int run_backend(Slot& s, const vsc_geom& g, double sharpen, const uchar4*
     return VSC_OK;
 }
 
+// PNG encoding (vsc_png.cuh): filtered stream, one deflate segment per PNG_SEG bytes of it, worst-case file bytes
+static size_t png_stream_bytes(int oh, int ow) { return (size_t)oh * (1 + 3 * (size_t)ow); }
+static size_t png_segments(int oh, int ow) { return (png_stream_bytes(oh, ow) + PNG_SEG - 1) / PNG_SEG; }
+static size_t png_capacity(int oh, int ow) { return 53 + png_stream_bytes(oh, ow) + 22 * png_segments(oh, ow); }
+// Encode the rgb24 frames (oh x ow) that fr[0..n) hold at l_out into PNG files at fr[i].l_png (device-accessible);
+// three launches on the leader's stream for the whole group.  The file sizes land in fr[i].h_png once the stream
+// has run.  stats: null, or the 3 debug counters of png_segment_kernel.
+static int run_png(Slot& lead, Slot* fr, int n, int oh, int ow, unsigned long long* stats) {
+    const size_t N = png_stream_bytes(oh, ow), nseg = png_segments(oh, ow);
+    if (nseg > (size_t)(1 << 30)) return fail(VSC_E_INVALID, "frame %dx%d too large for PNG output", ow, oh);
+    PngArgs a;
+    memset(&a, 0, sizeof a);
+    a.oh = oh; a.ow = ow; a.n = (long long)N; a.nseg = (int)nseg; a.stats = stats;
+    const size_t o_seg = align_up(N, 256), o_meta = o_seg + nseg * PNG_SEG_STRIDE,
+                 o_size = o_meta + align_up(nseg * sizeof(PngSegMeta), 256);
+    for (int i = 0; i < n; i++) {
+        if (fr[i].png_work.ensure(o_size + 256)) return VSC_E_NOMEM;
+        uint8_t* b = fr[i].png_work.as<uint8_t>();
+        a.img[i] = fr[i].l_out; a.dst[i] = fr[i].l_png;
+        a.filt[i] = b; a.seg[i] = b + o_seg; a.meta[i] = (PngSegMeta*)(b + o_meta); a.size[i] = (unsigned long long*)(b + o_size);
+    }
+    prof_begin(lead, "png_filter_kernel");
+    png_filter_kernel<<<dim3(oh, n), 256, 0, lead.stream>>>(a);
+    KCHECK(lead);
+    prof_begin(lead, "png_segment_kernel");
+    png_segment_kernel<<<dim3((unsigned)nseg, n), PNG_SEG_THREADS, PNG_SEG_SMEM, lead.stream>>>(a);
+    KCHECK(lead);
+    prof_begin(lead, "png_assemble_kernel");
+    png_assemble_kernel<<<dim3((unsigned)nseg, n), 256, 0, lead.stream>>>(a);
+    KCHECK(lead);
+    for (int i = 0; i < n; i++)
+        CU(cudaMemcpyAsync(fr[i].h_png, a.size[i], sizeof(unsigned long long), cudaMemcpyDeviceToHost, lead.stream));
+    return VSC_OK;
+}
+
 // ---- whole frame ----------------------------------------------------------------------------------
 static int ensure_frame_buffers(Slot& s, const vsc_geom& g, bool smoothing) {
     const size_t npx = (size_t)g.ss_h * g.ss_w;
@@ -832,6 +883,10 @@ static int enqueue_group(vsc_ctx* ctx, Slot* fr, int n, int dtype, const vsc_geo
     for (int i = 0; i < n; i++)
         if ((rc = run_backend(fr[i], g, p.sharpen, cur[2 * i], cur[2 * i + 1], fr[i].l_out, fr[i].l_layout,
                                   fr[i].l_pixfmt, fr[i].l_matrix))) return rc;
+    if (lead.l_encode == VSC_ENCODE_PNG) {
+        int oh, ow;
+        if ((rc = vsc_layout_shape(lead.l_layout, g.height, g.width, &oh, &ow)) || (rc = run_png(lead, fr, n, oh, ow, nullptr))) return rc;
+    }
     CU(cudaEventRecord(lead.ev1, lead.stream));
     for (int i = 0; i < n; i++)
         CU(cudaMemcpyAsync(fr[i].h_scalars, fr[i].scalars.p, sizeof(FrameScalars), cudaMemcpyDeviceToHost, lead.stream));
@@ -845,6 +900,13 @@ static void CUDART_CB on_submission_done(void* p) {       // runs on a driver th
         lead->done = true;
     }
     lead->owner->cv.notify_all();
+}
+
+// copies of the submission's outputs into caller-owned host buffers
+static int enqueue_d2h(Slot* fr, int n) {
+    for (int i = 0; i < n; i++)
+        if (fr[i].l_host_out) CU(cudaMemcpyAsync(fr[i].l_host_out, fr[i].l_copy_src, fr[i].l_out_bytes, cudaMemcpyDeviceToHost, fr[0].stream));
+    return VSC_OK;
 }
 
 static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const* rgb, const void* const* depth, int dtype,
@@ -862,27 +924,47 @@ static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const
     vsc_geom g;
     int rc;
     if ((rc = vsc_geometry(H, W, p, &g))) return rc;
-    const int layout = ctx->layout, pixfmt = ctx->pixfmt, matrix = ctx->matrix;
-    size_t nout;
+    const int layout = ctx->layout, pixfmt = ctx->pixfmt, matrix = ctx->matrix, encode = ctx->encode;
+    size_t nout, cap = 0;
     if ((rc = vsc_output_size(layout, pixfmt, H, W, &nout))) return rc;
+    if (encode == VSC_ENCODE_PNG) {
+        if (pixfmt != VSC_PIXFMT_RGB24) return fail(VSC_E_INVALID, "PNG output needs the rgb24 pixel format");
+        if ((rc = vsc_encoded_capacity(layout, encode, H, W, &cap))) return rc;
+    }
     CU(cudaSetDevice(ctx->device));
     const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype);
     for (int i = 0; i < n; i++) {
         Slot& s = fr[i];
         s.l_rgb = rgb[i]; s.l_depth = depth[i]; s.l_out = out[i]; s.l_host_out = nullptr; s.l_out_bytes = nout;
-        s.l_layout = layout; s.l_pixfmt = pixfmt; s.l_matrix = matrix;
+        s.l_layout = layout; s.l_pixfmt = pixfmt; s.l_matrix = matrix; s.l_encode = encode; s.l_png = nullptr;
         if (!device_io) {
             if (s.in_rgb.ensure(nrgb) || s.in_depth.ensure(ndepth) || s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
             CU(cudaMemcpyAsync(s.in_rgb.p, rgb[i], nrgb, cudaMemcpyHostToDevice, lead.stream));
             CU(cudaMemcpyAsync(s.in_depth.p, depth[i], ndepth, cudaMemcpyHostToDevice, lead.stream));
             s.l_rgb = s.in_rgb.as<uint8_t>(); s.l_depth = s.in_depth.p; s.l_out = s.out_sbs.as<uint8_t>();
-            s.l_host_out = out[i];
+            s.l_host_out = out[i]; s.l_copy_src = s.l_out;
+        }
+        if (encode == VSC_ENCODE_PNG) {
+            // the frame goes to the slot's own buffer, the file to the caller's: page-locked host memory is written by
+            // the device directly (only the file's bytes cross the bus); a pageable one gets the capacity after the run
+            if (device_io) {
+                if (s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
+                s.l_png = out[i]; s.l_out = s.out_sbs.as<uint8_t>();
+            } else {
+                cudaPointerAttributes at;
+                if (cudaPointerGetAttributes(&at, out[i]) == cudaSuccess && at.type == cudaMemoryTypeHost && at.devicePointer) {
+                    s.l_png = (uint8_t*)at.devicePointer; s.l_host_out = nullptr;
+                } else {
+                    cudaGetLastError();
+                    if (s.png_stage.ensure(cap)) return VSC_E_NOMEM;
+                    s.l_png = s.png_stage.as<uint8_t>(); s.l_copy_src = s.l_png; s.l_out_bytes = cap;
+                }
+            }
         }
     }
     rc = enqueue_group(ctx, fr, n, dtype, g, *p);
+    if (!rc) rc = enqueue_d2h(fr, n);
     if (rc) { cudaStreamSynchronize(lead.stream); return rc; }
-    for (int i = 0; i < n; i++)
-        if (fr[i].l_host_out) CU(cudaMemcpyAsync(fr[i].l_host_out, fr[i].l_out, nout, cudaMemcpyDeviceToHost, lead.stream));
     {
         std::lock_guard<std::mutex> lk(ctx->mu);
         lead.done = false;
@@ -944,9 +1026,8 @@ extern "C" int vsc_wait(vsc_ctx* ctx, int slot) {
         vsc_geom g;
         int rc = vsc_geometry(lead.l_H, lead.l_W, &lead.l_p, &g);
         if (!rc) rc = enqueue_group(ctx, fr, n, lead.l_dtype, g, lead.l_p);
+        if (!rc) rc = enqueue_d2h(fr, n);
         if (rc) { lead.busy = false; return rc; }
-        for (int i = 0; i < n; i++)
-            if (fr[i].l_host_out) CU(cudaMemcpyAsync(fr[i].l_host_out, fr[i].l_out, fr[i].l_out_bytes, cudaMemcpyDeviceToHost, lead.stream));
     }
     lead.busy = false;
     if (overflow) return fail(VSC_E_NOMEM, "hole-filling scratch overflow persisted");
@@ -1050,8 +1131,37 @@ extern "C" int vsc_set_pixfmt(vsc_ctx* ctx, int pixfmt, int matrix) {
     if (!ctx) return fail(VSC_E_INVALID, "null context");
     if (pixfmt < VSC_PIXFMT_RGB24 || pixfmt > VSC_PIXFMT_YUV420P10LE) return fail(VSC_E_INVALID, "unknown pixel format %d", pixfmt);
     if (matrix < VSC_MATRIX_BT709 || matrix > VSC_MATRIX_BT601) return fail(VSC_E_INVALID, "unknown yuv matrix %d", matrix);
+    if (ctx->encode == VSC_ENCODE_PNG && pixfmt != VSC_PIXFMT_RGB24)
+        return fail(VSC_E_INVALID, "PNG output needs the rgb24 pixel format: set the encoding to none first");
     ctx->pixfmt = pixfmt;
     ctx->matrix = matrix;
+    return VSC_OK;
+}
+
+extern "C" int vsc_encoded_capacity(int layout, int encode, int H, int W, size_t* bytes) {
+    if (!bytes) return fail(VSC_E_INVALID, "null argument");
+    if (encode == VSC_ENCODE_NONE) return vsc_output_size(layout, VSC_PIXFMT_RGB24, H, W, bytes);
+    if (encode != VSC_ENCODE_PNG) return fail(VSC_E_INVALID, "unknown encoding %d", encode);
+    int oh, ow, rc;
+    if ((rc = vsc_layout_shape(layout, H, W, &oh, &ow))) return rc;
+    *bytes = png_capacity(oh, ow);
+    return VSC_OK;
+}
+extern "C" int vsc_set_encode(vsc_ctx* ctx, int encode) {
+    if (!ctx) return fail(VSC_E_INVALID, "null context");
+    if (encode != VSC_ENCODE_NONE && encode != VSC_ENCODE_PNG) return fail(VSC_E_INVALID, "unknown encoding %d", encode);
+    if (encode == VSC_ENCODE_PNG && ctx->pixfmt != VSC_PIXFMT_RGB24)
+        return fail(VSC_E_INVALID, "PNG output needs the rgb24 pixel format");
+    ctx->encode = encode;
+    return VSC_OK;
+}
+extern "C" int vsc_encoded_bytes(vsc_ctx* ctx, int slot, int index, size_t* bytes) {
+    Slot* fr = group_lead(ctx, slot);
+    if (!fr || !bytes) return fail(VSC_E_INVALID, "bad argument");
+    if (fr->busy) return fail(VSC_E_STATE, "slot %d still has frames in flight; call vsc_wait first", slot);
+    if (index < 0 || index >= fr->nfr) return fail(VSC_E_INVALID, "frame %d is not part of slot %d's last submission", index, slot);
+    if (fr[index].l_encode != VSC_ENCODE_PNG) return fail(VSC_E_STATE, "slot %d's last submission was not encoded", slot);
+    *bytes = (size_t)*fr[index].h_png;
     return VSC_OK;
 }
 
@@ -1353,6 +1463,37 @@ extern "C" int vsc_depth_post_device(vsc_ctx* ctx, int slot, const float* d_dept
     CU(cudaSetDevice(ctx->device));
     return enqueue_depth_post(ctx, *fr, fr->stream, d_depth, h, w, H, W, bits, d_out);
 }
+extern "C" int vsc_stage_png(vsc_ctx* ctx, const uint8_t* rgb, int H, int W, uint8_t* out, size_t capacity, size_t* bytes) {
+    STAGE_BEGIN();
+    if (!rgb || !out || !bytes || H < 1 || W < 1) return fail(VSC_E_INVALID, "bad argument");
+    if ((long long)W * 3 + 1 > (1ll << 31) - 1) return fail(VSC_E_INVALID, "frame width %d too large for PNG output", W);
+    const size_t cap = png_capacity(H, W), nin = (size_t)H * W * 3;
+    if (capacity < cap) return fail(VSC_E_INVALID, "output capacity %zu is below vsc_encoded_capacity (%zu)", capacity, cap);
+    Tmp din, dout;
+    if (din.alloc(nin) || dout.alloc(cap) || s.png_stats.ensure(3 * sizeof(unsigned long long))) return VSC_E_NOMEM;
+    CU(cudaMemcpyAsync(din.p, rgb, nin, cudaMemcpyHostToDevice, s.stream));
+    CU(cudaMemsetAsync(s.png_stats.p, 0, 3 * sizeof(unsigned long long), s.stream));
+    s.l_out = (uint8_t*)din.p;
+    s.l_png = (uint8_t*)dout.p;
+    int rc = run_png(s, &s, 1, H, W, s.png_stats.as<unsigned long long>());
+    if (rc) { cudaStreamSynchronize(s.stream); return rc; }
+    CU(cudaStreamSynchronize(s.stream));
+    *bytes = (size_t)*s.h_png;
+    CU(cudaMemcpyAsync(out, dout.p, *bytes, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaStreamSynchronize(s.stream));
+    s.l_out = nullptr;
+    s.l_png = nullptr;
+    return VSC_OK;
+}
+extern "C" int vsc_debug_png_stats(vsc_ctx* ctx, unsigned long long* out) {
+    if (!ctx || !out) return fail(VSC_E_INVALID, "bad argument");
+    Slot& s = ctx->slots[0];
+    if (!s.png_stats.p) return fail(VSC_E_STATE, "no vsc_stage_png call on this context yet");
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaMemcpy(out, s.png_stats.p, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    return VSC_OK;
+}
+
 extern "C" int vsc_stage_depth_post(vsc_ctx* ctx, const float* depth, int h, int w, int H, int W, int bits, void* out, int* ok) {
     STAGE_BEGIN();
     int rc = depth_post_args_ok(depth, out, h, w, H, W, bits);

@@ -18,6 +18,8 @@ There is no CPU path: `--cpu` is refused.
 side-by-side (default), half side-by-side, top-bottom, half top-bottom or a red-cyan anaglyph (INTEGRATION.md).
 `--pixfmt` / `--matrix` (or the top-level keys "sbs_pixfmt" / "sbs_matrix") hand the raw sink encoder-ready YUV 4:2:0
 (yuv420p, yuv420p10le; BT.709 or BT.601, limited range) instead of rgb24; a YUV format needs `--raw-sink`.
+`--png-encoder gpu` (or the top-level key "sbs_png_encoder") has the GPU encode sbs_*.png and the savers write its bytes
+verbatim; the default `cv2` encodes on the saver threads with cv2.imencode.
 """
 from __future__ import annotations
 
@@ -33,6 +35,7 @@ from pathlib import Path
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 from vsc_b200.stereo_core import LAYOUTS, MATRICES, PIXFMTS  # noqa: E402
+from vsc_b200.workflow import PNG_ENCODERS  # noqa: E402
 
 GPU_ERROR_EXIT_CODE = 100      # reference: sbs_generator.py:41
 
@@ -69,6 +72,9 @@ def build_parser() -> ArgumentParser:
                         'yuv420p10le (I420, limited range) need --raw-sink')
     p.add_argument('--matrix', choices=MATRICES, default=None,
                    help='YUV matrix of the yuv420 formats (default: config.json "sbs_matrix", else bt709)')
+    p.add_argument('--png-encoder', choices=PNG_ENCODERS, default=None,
+                   help='who encodes sbs_*.png (default: config.json "sbs_png_encoder", else cv2): cv2 on the CPU saver '
+                        'threads, or gpu (rgb24 only, not with --raw-sink)')
     return p
 
 
@@ -162,7 +168,7 @@ def open_raw_sink(path: str, pairs, layout: str, pixfmt: str = 'rgb24', matrix: 
 
 def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int, io_threads: int, free_space_mode: str,
                   no_interactive: bool, progress=None, sink=None, sink_index=None, group: int = 4, gen=None,
-                  layout: str = 'sbs', pixfmt: str = 'rgb24', matrix: str = 'bt709') -> int:
+                  layout: str = 'sbs', pixfmt: str = 'rgb24', matrix: str = 'bt709', png_encoder: str = 'cv2') -> int:
     """Run `pairs` [(frame_path, depth_path, frame_num)] through one GPU.  Returns frames written.
 
     The pipeline the benchmark times: `slots` frame slots of `group` frames each.  A slot is filled by the loader
@@ -171,7 +177,8 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
     pool (bounded backlog) and become visible in frame order through the InOrderPublisher.
     With `sink` (a RawFrameSink shared by all GPUs of the process) frames go to it at position
     `sink_index[frame_num]` instead of into sbs_<n>.png.  `layout`, `pixfmt` and `matrix` set the output of a generator
-    made here (a YUV pixfmt only with a sink)."""
+    made here (a YUV pixfmt only with a sink).  png_encoder='gpu' has that generator encode the PNG files (a caller's
+    generator must then have encode='png'), and the savers write its bytes as they are."""
     import cv2
     import numpy as np
     from vsc_b200 import StereoGenerator
@@ -180,7 +187,7 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
     own_gen = gen is None         # a caller may pass a warm generator (n_slots >= slots, group_size >= group) and keep it
     if own_gen:
         gen = StereoGenerator(f'cuda:{device_index}', n_slots=slots, group_size=group, layout=layout, pixfmt=pixfmt,
-                              matrix=matrix)
+                              matrix=matrix, encode='png' if png_encoder == 'gpu' else None)
     loaders = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='load')
     savers = ThreadPoolExecutor(max_workers=io_threads, thread_name_prefix='save')
     backlog = threading.BoundedSemaphore(max(2 * io_threads, group))     # frames waiting for / inside the savers
@@ -212,9 +219,12 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
                 staged = InOrderPublisher.staged_path(final)
                 for attempt in range(3):        # reference: 3 retries, 60 s apart (sbs_generator.py:241-262)
                     try:
-                        ok, buf = cv2.imencode('.png', cv2.cvtColor(sbs, cv2.COLOR_RGB2BGR))
-                        if not ok:
-                            raise IOError(f'PNG encode failed for {final}')
+                        if gen.encode == 'png':
+                            buf = sbs                       # already the PNG file
+                        else:
+                            ok, buf = cv2.imencode('.png', cv2.cvtColor(sbs, cv2.COLOR_RGB2BGR))
+                            if not ok:
+                                raise IOError(f'PNG encode failed for {final}')
                         with open(staged, 'wb') as f:
                             f.write(buf.tobytes())
                         InOrderPublisher.mark_ready(final)
@@ -328,7 +338,7 @@ def main(argv=None) -> int:
         print(f'ERROR: Workflow directory not found: {args.workflow_path}')
         return 0
     ConfigError, get_path, load_config = _load_config_api()
-    from vsc_b200.workflow import LayoutError, config_layout, config_pixfmt
+    from vsc_b200.workflow import LayoutError, config_layout, config_pixfmt, config_png_encoder
     try:
         config = load_config(args.workflow_path)
     except ConfigError as e:
@@ -350,10 +360,17 @@ def main(argv=None) -> int:
     try:
         layout = args.layout or config_layout(config)
         cfg_pixfmt, cfg_matrix = config_pixfmt(config)
+        png_encoder = args.png_encoder or config_png_encoder(config)
     except LayoutError as e:
         print(f'ERROR: {e}')
         return 2
     pixfmt, matrix = args.pixfmt or cfg_pixfmt, args.matrix or cfg_matrix
+    if png_encoder == 'gpu' and args.raw_sink:
+        print('ERROR: --png-encoder gpu encodes sbs_*.png files; the raw sink takes raw frames (drop one of the two)')
+        return 2
+    if png_encoder == 'gpu' and pixfmt != 'rgb24':
+        print(f'ERROR: --png-encoder gpu writes rgb24 PNG files, not pixel format {pixfmt}')
+        return 2
     if pixfmt != 'rgb24' and not args.raw_sink:
         print(f'ERROR: pixel format {pixfmt} is for the raw sink only (--raw-sink); sbs_*.png files are rgb24')
         return 2
@@ -395,7 +412,8 @@ def main(argv=None) -> int:
         print(f'Parameters: disparity={params.max_disparity}, convergence={params.convergence}, '
               f'super_sampling={params.super_sampling}, edge_softness={params.edge_softness}, '
               f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}, layout={layout}'
-              + (f', pixfmt={pixfmt}, matrix={matrix}' if pixfmt != 'rgb24' else ''))
+              + (f', pixfmt={pixfmt}, matrix={matrix}' if pixfmt != 'rgb24' else '')
+              + (', png_encoder=gpu' if png_encoder == 'gpu' else ''))
 
     finals = [str(output_dir / f'sbs_{p[2]}.png') for p in pairs]
 
@@ -440,7 +458,7 @@ def main(argv=None) -> int:
             if t:
                 t.start()
             n = process_shard(mine, output_dir, params, local_rank, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                              group=args.group, layout=layout)
+                              group=args.group, layout=layout, png_encoder=png_encoder)
             barrier()
             if t:
                 pub.stop()
@@ -455,7 +473,7 @@ def main(argv=None) -> int:
             t.start()
             if g == 1:
                 n = process_shard(pairs, output_dir, params, 0, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                                  sink, sink_index, args.group, layout=layout, pixfmt=pixfmt, matrix=matrix)
+                                  sink, sink_index, args.group, layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder)
             else:
                 # one worker thread per GPU; each owns a StereoGenerator (its own CUDA context state, streams, pinned ring)
                 results = [0] * g
@@ -465,7 +483,7 @@ def main(argv=None) -> int:
                     try:
                         results[k] = process_shard(shard_items(pairs, g, k), output_dir, params, k, args.slots, args.io_threads,
                                                    free_space_mode, args.no_interactive, progress, sink, sink_index, args.group,
-                                                   layout=layout, pixfmt=pixfmt, matrix=matrix)
+                                                   layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder)
                     except BaseException as e:   # noqa: BLE001
                         errors.append(e)
                 ths = [threading.Thread(target=work, args=(k,)) for k in range(g)]

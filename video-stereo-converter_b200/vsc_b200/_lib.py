@@ -18,6 +18,7 @@ DEPTH_U8, DEPTH_U16, DEPTH_F32 = 0, 1, 2
 LAYOUT_SBS, LAYOUT_HALF_SBS, LAYOUT_TB, LAYOUT_HALF_TB, LAYOUT_ANAGLYPH = 0, 1, 2, 3, 4
 PIXFMT_RGB24, PIXFMT_YUV420P, PIXFMT_YUV420P10LE = 0, 1, 2
 MATRIX_BT709, MATRIX_BT601 = 0, 1
+ENCODE_NONE, ENCODE_PNG = 0, 1
 GPU_ERROR_EXIT_CODE = 100      # sbs_generator.py:41
 
 EXPORTS = [
@@ -30,6 +31,7 @@ EXPORTS = [
     'vsc_set_profiling', 'vsc_slot_kernel_times', 'vsc_timer_begin', 'vsc_timer_end', 'vsc_debug_fetch',
     'vsc_debug_telea_state', 'vsc_debug_telea_stats', 'vsc_debug_set_telea_capacity', 'vsc_debug_selftest',
     'vsc_layout_shape', 'vsc_set_layout', 'vsc_output_size', 'vsc_set_pixfmt',
+    'vsc_set_encode', 'vsc_encoded_capacity', 'vsc_encoded_bytes', 'vsc_stage_png', 'vsc_debug_png_stats',
 ]
 
 
@@ -118,6 +120,11 @@ def load():
     lib.vsc_set_layout.argtypes = [vp, i]
     lib.vsc_output_size.argtypes = [i, i, i, i, C.POINTER(C.c_size_t)]
     lib.vsc_set_pixfmt.argtypes = [vp, i, i]
+    lib.vsc_set_encode.argtypes = [vp, i]
+    lib.vsc_encoded_capacity.argtypes = [i, i, i, i, C.POINTER(C.c_size_t)]
+    lib.vsc_encoded_bytes.argtypes = [vp, i, i, C.POINTER(C.c_size_t)]
+    lib.vsc_stage_png.argtypes = [vp, vp, i, i, vp, C.c_size_t, C.POINTER(C.c_size_t)]
+    lib.vsc_debug_png_stats.argtypes = [vp, C.POINTER(C.c_ulonglong)]
     if lib.vsc_abi_version() != 1:
         raise ImportError('libvsc_b200.so ABI version mismatch')
     _lib = lib

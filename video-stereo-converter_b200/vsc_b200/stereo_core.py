@@ -11,6 +11,8 @@ Additions that the reference does not have (used by the frame loop in sbs_genera
 `output_shape(layout, h, w)` instead of the side-by-side [h, 2w, 3].  Output pixel formats
 (`StereoGenerator(..., pixfmt='yuv420p10le', matrix='bt709')`, `PIXFMTS`, `MATRICES`, `output_dtype`): the YUV formats
 return the I420 planes of that frame as one [rows * 3 // 2, cols] array, the shape cv2's COLOR_RGB2YUV_I420 uses.
+PNG output (`StereoGenerator(..., encode='png')`, `ENCODINGS`, `encoded_capacity`): every output path returns the PNG file
+of the rgb24 frame, encoded on the GPU, as a 1-D uint8 array of exactly the file's bytes.
 """
 from __future__ import annotations
 
@@ -81,6 +83,29 @@ def matrix_code(matrix: str) -> int:
 def output_dtype(pixfmt: str) -> np.dtype:
     """Element type of the frames of a pixel format: uint16 (value in the low 10 bits) for yuv420p10le, else uint8."""
     return np.dtype(np.uint16 if pixfmt_code(pixfmt) == _lib.PIXFMT_YUV420P10LE else np.uint8)
+
+
+# encoded outputs (include/vsc_b200.h VSC_ENCODE_*): name -> C enum; None (raw frames) is VSC_ENCODE_NONE
+ENCODINGS = ('png',)
+
+
+def encode_code(encode: Optional[str]) -> int:
+    """C enum of an encoding name (None: raw frames); ValueError for anything else."""
+    if encode is None:
+        return _lib.ENCODE_NONE
+    if encode not in ENCODINGS:
+        raise ValueError(f'unknown encoding {encode!r} (None or one of {", ".join(ENCODINGS)})')
+    return ENCODINGS.index(encode) + 1
+
+
+def encoded_capacity(layout: str, h: int, w: int) -> int:
+    """Worst-case bytes of the PNG file of the frame `layout` makes of an h x w input (the size an output buffer of an
+    encoding generator must have).  ValueError for an unknown layout or a size it cannot take."""
+    n = C.c_size_t()
+    rc = _lib.load().vsc_encoded_capacity(layout_code(layout), _lib.ENCODE_PNG, int(h), int(w), C.byref(n))
+    if rc != _lib.VSC_OK:
+        raise ValueError((_lib.load().vsc_last_error() or b'').decode('utf-8', 'replace'))
+    return int(n.value)
 
 
 def output_shape(layout: str, h: int, w: int, pixfmt: str = 'rgb24') -> Tuple[int, ...]:
@@ -228,18 +253,20 @@ class StereoGenerator:
     `n_slots` frames can be in flight through `submit` / `collect` for the driver loop.
     `layout` (one of LAYOUTS, default the reference's 'sbs') sets the shape of every frame this generator returns, and
     `pixfmt` (one of PIXFMTS, default 'rgb24') with `matrix` (one of MATRICES, for the YUV formats) its pixel format.
+    `encode='png'` (rgb24 only) makes every output path return the frame's PNG file as a 1-D uint8 array instead.
     """
     _DEFAULT_PARAMS = StereoParams()
 
     def __init__(self, device: str, n_slots: int = 1, group_size: int = 1, layout: str = 'sbs', pixfmt: str = 'rgb24',
-                 matrix: str = 'bt709') -> None:
+                 matrix: str = 'bt709', encode: Optional[str] = None) -> None:
         self.device = device
-        code, fcode, mcode = layout_code(layout), pixfmt_code(pixfmt), matrix_code(matrix)
+        code, fcode, mcode, ecode = layout_code(layout), pixfmt_code(pixfmt), matrix_code(matrix), encode_code(encode)
         self._ctx = _lib.Context(_parse_device(device), n_slots, group_size)
         self._lib = _lib.load()
         _lib.check(self._lib.vsc_set_layout(self._ctx.handle, code))
         _lib.check(self._lib.vsc_set_pixfmt(self._ctx.handle, fcode, mcode))
-        self.layout, self.pixfmt, self.matrix = layout, pixfmt, matrix
+        _lib.check(self._lib.vsc_set_encode(self._ctx.handle, ecode))
+        self.layout, self.pixfmt, self.matrix, self.encode = layout, pixfmt, matrix, encode
         self.n_slots, self.group_size = n_slots, group_size
         self._pending = [None] * n_slots        # per slot: number of frames in flight
         # pinned staging per (slot, frame index within the slot's group): (key, rgb, depth, out) PinnedBuffers
@@ -248,14 +275,15 @@ class StereoGenerator:
     # -- reference API ---------------------------------------------------------------------------
     def process_frame(self, rgb: np.ndarray, depth: np.ndarray, params: StereoParams | None = None) -> np.ndarray:
         """Process a single frame to a side-by-side stereo image (left | right), uint8 [H, 2W, 3]
-        (with another layout or pixel format: output_shape(layout, H, W, pixfmt) of output_dtype(pixfmt))."""
+        (with another layout or pixel format: output_shape(layout, H, W, pixfmt) of output_dtype(pixfmt); with
+        encode='png': the PNG file's bytes)."""
         p = params or self._DEFAULT_PARAMS
         rgb_c, depth_c, code = self._check_inputs(rgb, depth)
         h, w = rgb_c.shape[:2]
-        out = np.empty(self.output_shape(h, w), self.output_dtype)
+        out = np.empty(*self._out_spec(h, w))
         _lib.check(self._lib.vsc_process_frame(self._ctx.handle, _lib.ptr(rgb_c), _lib.ptr(depth_c), code, h, w,
                                                C.byref(_lib.make_params(p)), _lib.ptr(out)))
-        return out
+        return out[:self.encoded_bytes(0)].copy() if self.encode else out
 
     # -- asynchronous pipeline ---------------------------------------------------------------------
     def pinned_inputs(self, slot: int, h: int, w: int, depth_dtype=np.uint8, index: int = 0):
@@ -270,7 +298,7 @@ class StereoGenerator:
                 for b in pin[1:]:
                     b.free()
             pin = (key, _lib.PinnedBuffer((h, w, 3), np.uint8), _lib.PinnedBuffer((h, w), depth_dtype),
-                   _lib.PinnedBuffer(self.output_shape(h, w), self.output_dtype))
+                   _lib.PinnedBuffer(*self._out_spec(h, w)))
             self._pinned[slot][index] = pin
         return pin[1].array, pin[2].array
 
@@ -352,6 +380,8 @@ class StereoGenerator:
             self._pending[slot] = None
             getattr(self, '_held', {}).pop(slot, None)
         outs = [self._pinned[slot][i][3].array for i in range(n)]
+        if self.encode:
+            outs = [o[:self.encoded_bytes(slot, i)] for i, o in enumerate(outs)]
         if copy:
             outs = [o.copy() for o in outs]
         return outs[0] if n == 1 else outs
@@ -359,7 +389,8 @@ class StereoGenerator:
     def submit_device(self, slot: int, d_rgb: int, d_depth: int, depth_dtype, h: int, w: int, d_out: int,
                       params: StereoParams | None = None) -> None:
         """Device-resident variant: raw device pointers (e.g. torch tensor .data_ptr()), no copies.  d_out must hold
-        output_shape(h, w) of output_dtype (self.output_shape, self.output_dtype)."""
+        output_shape(h, w) of output_dtype (self.output_shape, self.output_dtype); with encode='png', encoded_capacity
+        bytes, of which encoded_bytes(slot) are the file once the slot has been waited for."""
         p = params or self._DEFAULT_PARAMS
         _lib.check(self._lib.vsc_submit_device(self._ctx.handle, slot, C.c_void_p(d_rgb), C.c_void_p(d_depth),
                                                _lib.depth_code(depth_dtype), h, w, C.byref(_lib.make_params(p)),
@@ -374,6 +405,12 @@ class StereoGenerator:
         _lib.check(self._lib.vsc_submit_device_group(
             self._ctx.handle, slot, n, vp(*[t[0] for t in triples]), vp(*[t[1] for t in triples]), _lib.depth_code(depth_dtype),
             h, w, C.byref(_lib.make_params(p)), vp(*[t[2] for t in triples])))
+
+    def encoded_bytes(self, slot: int, index: int = 0) -> int:
+        """Bytes of the PNG file of frame `index` of the slot's last completed submission (encode='png')."""
+        n = C.c_size_t()
+        _lib.check(self._lib.vsc_encoded_bytes(self._ctx.handle, slot, index, C.byref(n)))
+        return int(n.value)
 
     def wait(self, slot: int) -> None:
         _lib.check(self._lib.vsc_wait(self._ctx.handle, slot))
@@ -508,7 +545,23 @@ class StereoGenerator:
         self.pixfmt, self.matrix = pixfmt, matrix
         self._release_pinned()
 
+    def set_encode(self, encode: Optional[str]) -> None:
+        """Switch the encoding of frames submitted from now on (None: raw frames, 'png').  Every slot must be collected,
+        as for set_layout."""
+        ecode = encode_code(encode)
+        if any(x is not None for x in self._pending):
+            raise RuntimeError('collect every slot before changing the encoding')
+        _lib.check(self._lib.vsc_set_encode(self._ctx.handle, ecode))
+        self.encode = encode
+        self._release_pinned()
+
     # -- helpers -----------------------------------------------------------------------------------
+    def _out_spec(self, h: int, w: int):
+        """(shape, dtype) of the output buffer of one frame: the frame, or with an encoding its worst-case file."""
+        if self.encode:
+            return (encoded_capacity(self.layout, h, w),), np.dtype(np.uint8)
+        return self.output_shape(h, w), self.output_dtype
+
     def output_shape(self, h: int, w: int) -> Tuple[int, ...]:
         """Shape of the frames this generator returns for h x w inputs."""
         return output_shape(self.layout, h, w, self.pixfmt)

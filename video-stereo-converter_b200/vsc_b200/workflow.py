@@ -9,7 +9,8 @@ One key is this implementation's own: the optional top-level "sbs_layout" (outpu
 stereo_core.LAYOUTS, default "sbs").  It sits at the top level because the reference's validator accepts extra
 top-level keys while the reference builds StereoParams from the whole `stereo` block.  So do the optional
 "sbs_pixfmt" (pixel format of the frames, one of stereo_core.PIXFMTS, default "rgb24") and "sbs_matrix" (YUV matrix, one
-of stereo_core.MATRICES, default "bt709").
+of stereo_core.MATRICES, default "bt709"), and "sbs_png_encoder" (who encodes sbs_*.png, one of PNG_ENCODERS, default
+"cv2").
 """
 from __future__ import annotations
 
@@ -21,6 +22,9 @@ STEREO_KEYS = ('max_disparity', 'convergence', 'super_sampling', 'edge_softness'
 DIR_KEYS = ('frames', 'depth_maps', 'sbs')
 LAYOUT_KEY = 'sbs_layout'
 PIXFMT_KEY, MATRIX_KEY = 'sbs_pixfmt', 'sbs_matrix'
+PNG_ENCODER_KEY = 'sbs_png_encoder'
+# who encodes sbs_*.png: 'cv2' (cv2.imencode on the saver threads) or 'gpu' (the library's PNG encoding, written verbatim)
+PNG_ENCODERS = ('cv2', 'gpu')
 
 
 class ConfigError(Exception):
@@ -28,8 +32,8 @@ class ConfigError(Exception):
 
 
 class LayoutError(ConfigError):
-    """One of the optional output keys ("sbs_layout", "sbs_pixfmt", "sbs_matrix") holds something other than a name
-    it takes."""
+    """One of the optional output keys ("sbs_layout", "sbs_pixfmt", "sbs_matrix", "sbs_png_encoder") holds something
+    other than a name it takes."""
 
 
 def config_layout(cfg: Dict) -> str:
@@ -51,6 +55,14 @@ def config_pixfmt(cfg: Dict):
             raise LayoutError(f"Invalid '{key}' {v!r} (expected one of {', '.join(names)})")
         out.append(v)
     return tuple(out)
+
+
+def config_png_encoder(cfg: Dict) -> str:
+    """The PNG encoder a config asks for: top-level "sbs_png_encoder", default 'cv2'."""
+    v = cfg.get(PNG_ENCODER_KEY, 'cv2')
+    if v not in PNG_ENCODERS:
+        raise LayoutError(f"Invalid '{PNG_ENCODER_KEY}' {v!r} (expected one of {', '.join(PNG_ENCODERS)})")
+    return v
 
 
 def load_config(workflow_path) -> Dict:
@@ -75,6 +87,7 @@ def load_config(workflow_path) -> Dict:
             raise ConfigError(f"Missing or invalid 'stereo.{k}' (expected float)")
     config_layout(cfg)
     config_pixfmt(cfg)
+    config_png_encoder(cfg)
     return cfg
 
 
