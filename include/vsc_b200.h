@@ -233,6 +233,42 @@ int vsc_stage_png(vsc_ctx *ctx, const uint8_t *rgb, int height, int width, uint8
 int vsc_stage_depth_post(vsc_ctx *ctx, const float *depth, int h, int w, int H, int W, int bits, void *out, int *ok);
 int vsc_depth_post_device(vsc_ctx *ctx, int slot, const float *d_depth, int h, int w, int H, int W, int bits, void *d_out);
 
+/* -------- temporal depth stabilisation (no reference counterpart) ------------------------------ */
+/* The depth map of frame t is filtered over the maps D_j of its window lo <= j <= hi (t-k <= lo, hi <= t+k, k = radius
+ * in 0..8), all uint8 or uint16 (M = 255 / 65535) of one size H x W, n = H*W:
+ *   sums     S_j = sum D_j, Q_j = sum D_j^2, P_tj = sum D_t D_j, exact (u64);  in 128-bit integers
+ *            cov = n P_tj - S_t S_j, var_j = n Q_j - S_j^2, var_t = n Q_t - S_t^2, each then rounded to double
+ *            (nearest, ties to even)
+ *   cut      neighbour j is cut if var_j <= 0, var_t <= 0, cov <= 0, 2 cov^2 < var_j var_t (double, in that order; r^2 < 1/2)
+ *            or a > 16; a cut excludes every neighbour farther out on its side too (a scene boundary), and so does a
+ *            frame the caller has no map for (clip ends, gaps)
+ *   align    D_t ~ a D_j + b in IEEE double, no contraction:  a = cov / var_j,  b = (S_t - a S_j) / n,
+ *            A = rint(a 65536), B = rint(b 65536) (int64, half to even),
+ *            E_j = clamp((A D_j + B + 32768) >> 16, 0, M) (arithmetic shift);  E_t = D_t
+ *   weights  w[m][d] = (float) exp(-0.5 m^2 / k^2 - 0.5 d^2 / sigma^2) in double (m = 0..k, d = 0..255; the m term is 0
+ *            for m = 0), sigma in (0, 64] in 8-bit depth units; neighbour j weighs w[|j - t|][min(d, 255)] with
+ *            d = |E_j - D_t| (uint8) or |E_j - D_t| >> 8 (uint16)
+ *   output   f32 (sum_j w E_j) / (sum_j w), j ascending from lo to hi, centre included (w[0][0] = 1), every product, sum
+ *            and the quotient rounded to nearest f32
+ * Each output frame is a pure function of its rgb and its window: no state crosses submissions. */
+/* vsc_submit_group with temporally filtered depth: frame i of the n frames is depth[first + i], so they are consecutive
+ * clip frames, and the window of frame i is every plane the caller passes within radius of it (pass fewer planes at the
+ * ends of a clip or at a gap).  The planes a submission uses (depth[first - radius .. first + n - 1 + radius], clipped to
+ * the n_depth given) are copied into the slot's window buffer; two kernels then write each frame's f32 map, which the
+ * pipeline takes as VSC_DEPTH_F32 depth.  Layouts, pixel formats and encodings apply as with vsc_submit_group.
+ * radius 0 is vsc_submit_group (any dtype); with radius > 0 dtype must be u8 or u16 (VSC_E_INVALID otherwise). */
+int vsc_submit_window(vsc_ctx *ctx, int slot, int n, const uint8_t *const *rgb, int n_depth, const void *const *depth,
+                      int first, int dtype, int height, int width, int radius, double sigma, const vsc_params *p,
+                      uint8_t *const *out);
+/* the same with device pointers (like vsc_submit_device_group: enqueues only) */
+int vsc_submit_device_window(vsc_ctx *ctx, int slot, int n, const uint8_t *const *d_rgb, int n_depth,
+                             const void *const *d_depth, int first, int dtype, int height, int width, int radius,
+                             double sigma, const vsc_params *p, uint8_t *const *d_out);
+/* The filter alone on host planes (synchronous): frame t of depth[0 .. n_depth) -> out f32 [H][W]; *lo / *hi (may be
+ * NULL) = the window that survived the cut rule, as indices into depth. */
+int vsc_stage_temporal_depth(vsc_ctx *ctx, const void *const *depth, int n_depth, int t, int dtype, int height, int width,
+                             int radius, double sigma, float *out, int *lo, int *hi);
+
 /* -------- the module-level helpers that stereo_core.__all__ exports (stereo_core.py:22-29) ---- */
 /* normalize_depth (stereo_core.py:71-88) on n floats */
 int vsc_stage_normalize_f32(vsc_ctx *ctx, const float *in, size_t n, float *out);
@@ -270,6 +306,9 @@ int vsc_debug_selftest(vsc_ctx *ctx, int which, unsigned long long *mismatches);
 /* counters of the last vsc_stage_png call: out[0] segments whose lit/len code needed the 15-bit limit, out[1] segments
  * whose code-length code needed the 7-bit limit, out[2] segments written as stored blocks */
 int vsc_debug_png_stats(vsc_ctx *ctx, unsigned long long *out);
+/* the temporal filter's device conversion of a 128-bit integer to double on n values, two's complement, two words each
+ * (low word first) -> out[n] */
+int vsc_debug_i128_to_double(vsc_ctx *ctx, const uint64_t *words, int n, double *out);
 
 #ifdef __cplusplus
 }

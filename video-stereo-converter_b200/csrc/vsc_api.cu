@@ -23,6 +23,7 @@
 #include "../../include/vsc_b200.h"
 #include "vsc_march.cuh"
 #include "vsc_png.cuh"
+#include "vsc_temporal.cuh"
 
 using namespace vsc;
 
@@ -254,6 +255,11 @@ struct Slot {
     DevBuf png_work;    // PNG: filtered stream, segment blocks, segment metadata, file size
     DevBuf png_stage;   // PNG file of a submission whose host destination is pageable
     DevBuf png_stats;   // PNG debug counters (vsc_stage_png)
+    DevBuf tdepth;      // temporal filter: this frame's f32 depth plane (the pipeline's VSC_DEPTH_F32 input)
+    DevBuf twin, tsums, twtab;   // leader only: window planes, integer sums + surviving windows, weight table
+    int tw_k = -1; double tw_sigma = 0.0;   // key of the weight table in twtab
+    TemporalArgs l_temporal;             // leader only: the submission's temporal filter (k == 0: none)
+    int tw_jobs = 0;                     // leader only: its sums jobs
     FrameScalars* h_scalars = nullptr;   // pinned mirror
     unsigned long long* h_png = nullptr; // pinned: bytes of the PNG file of the last submission
     // table cache key
@@ -453,6 +459,10 @@ extern "C" void vsc_destroy(vsc_ctx* ctx) {
         s.png_work.release();
         s.png_stage.release();
         s.png_stats.release();
+        s.tdepth.release();
+        s.twin.release();
+        s.tsums.release();
+        s.twtab.release();
         for (cudaEvent_t e : s.pev) cudaEventDestroy(e);
         if (s.h_scalars) cudaFreeHost(s.h_scalars);
         if (s.h_png) cudaFreeHost(s.h_png);
@@ -819,6 +829,74 @@ static int run_png(Slot& lead, Slot* fr, int n, int oh, int ow, unsigned long lo
     return VSC_OK;
 }
 
+// ---- temporal depth filter (vsc_temporal.cuh) -----------------------------------------------------
+static bool temporal_args_ok(int radius, double sigma) { return radius >= 0 && radius <= TD_MAX_RADIUS && sigma > 0.0 && sigma <= 64.0; }
+// w[m][d] = (float) exp(-0.5 m^2 / k^2 - 0.5 d^2 / sigma^2) in double, the expression tests/temporal_oracle.py evaluates
+// with math.exp (the same libm); cached in the leader by (k, sigma).  Called while the slot is idle.
+static int ensure_weights(Slot& lead, int k, double sigma) {
+    if (lead.tw_k == k && lead.tw_sigma == sigma && lead.twtab.p) return VSC_OK;
+    std::vector<float> w((size_t)(k + 1) * 256);
+    for (int m = 0; m <= k; m++) {
+        const double tm = m == 0 ? 0.0 : 0.5 * (double)(m * m) / (double)(k * k);
+        for (int d = 0; d < 256; d++) w[(size_t)m * 256 + d] = (float)exp(-tm - 0.5 * (double)(d * d) / (sigma * sigma));
+    }
+    if (lead.twtab.ensure(w.size() * 4)) return VSC_E_NOMEM;
+    CU(cudaMemcpyAsync(lead.twtab.p, w.data(), w.size() * 4, cudaMemcpyHostToDevice, lead.stream));
+    CU(cudaStreamSynchronize(lead.stream));   // w is a temporary
+    lead.tw_k = k; lead.tw_sigma = sigma;
+    return VSC_OK;
+}
+// Copy the np window planes (host or device pointers) into the leader's window buffer, 16-byte aligned, and set up
+// the filter of frames f0 .. f0+n-1 into outs.  The weight table must be current (ensure_weights).
+static int stage_window(Slot& lead, const void* const* planes, int np, int f0, int n, int k, int dtype, int H, int W,
+                        bool device_io, float* const* outs) {
+    const long long npx = (long long)H * W;
+    const size_t bytes = (size_t)npx * depth_elem(dtype), stride = align_up(bytes, 16);
+    if (lead.twin.ensure(stride * np) || lead.tsums.ensure(TD_SUMS * 8 + 2 * TD_MAX_FRAMES * 4)) return VSC_E_NOMEM;
+    for (int j = 0; j < np; j++)
+        CU(cudaMemcpyAsync(lead.twin.as<uint8_t>() + j * stride, planes[j], bytes,
+                           device_io ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, lead.stream));
+    TemporalArgs& a = lead.l_temporal;
+    memset(&a, 0, sizeof a);
+    a.planes = lead.twin.as<uint8_t>(); a.stride = (long long)stride; a.npx = npx;
+    a.np = np; a.n = n; a.f0 = f0; a.k = k; a.maxv = dtype == VSC_DEPTH_U8 ? 255 : 65535;
+    int nj = 0;
+    for (int j = 0; j < np; j++) { a.ja[nj] = (signed char)j; a.jb[nj] = -1; nj++; }
+    for (int i = 0; i < n; i++)
+        for (int side = 0; side < 2; side++)
+            for (int m = 1; m <= k; m++) {
+                const int t = f0 + i, j = side ? t + m : t - m;
+                if (j < 0 || j >= np) continue;
+                a.ja[nj] = (signed char)t; a.jb[nj] = (signed char)j; a.jout[nj] = (short)(i * 2 * k + side * k + m - 1);
+                nj++;
+            }
+    a.sums = lead.tsums.as<unsigned long long>();
+    a.win = (int*)(lead.tsums.as<uint8_t>() + TD_SUMS * 8);
+    a.wtab = lead.twtab.as<float>();
+    for (int i = 0; i < n; i++) a.out[i] = outs[i];
+    lead.tw_jobs = nj;      // rows of the sums kernel's grid
+    return VSC_OK;
+}
+// the two launches of the filter staged by stage_window, on the leader's stream
+static int run_temporal(vsc_ctx* ctx, Slot& lead) {
+    const TemporalArgs& a = lead.l_temporal;
+    const int es = a.maxv == 255 ? 1 : 2, nj = lead.tw_jobs;
+    CU(cudaMemsetAsync(a.sums, 0, TD_SUMS * 8, lead.stream));
+    const long long nv = a.npx * es / 16;
+    const long long bx = std::max(1ll, std::min((nv + kThreads - 1) / kThreads, (long long)(8 * ctx->sm_count + nj - 1) / nj));
+    prof_begin(lead, "temporal_sums_kernel");
+    if (es == 1) temporal_sums_kernel<uint8_t><<<dim3((unsigned)bx, nj), kThreads, 0, lead.stream>>>(a);
+    else temporal_sums_kernel<uint16_t><<<dim3((unsigned)bx, nj), kThreads, 0, lead.stream>>>(a);
+    KCHECK(lead);
+    const long long nq = (a.npx + 3) / 4;
+    const long long fx = std::max(1ll, std::min((nq + kThreads - 1) / kThreads, (long long)(8 * ctx->sm_count + a.n - 1) / a.n));
+    prof_begin(lead, "temporal_filter_kernel");
+    if (es == 1) temporal_filter_kernel<uint8_t><<<dim3((unsigned)fx, a.n), kThreads, 0, lead.stream>>>(a);
+    else temporal_filter_kernel<uint16_t><<<dim3((unsigned)fx, a.n), kThreads, 0, lead.stream>>>(a);
+    KCHECK(lead);
+    return VSC_OK;
+}
+
 // ---- whole frame ----------------------------------------------------------------------------------
 static int ensure_frame_buffers(Slot& s, const vsc_geom& g, bool smoothing) {
     const size_t npx = (size_t)g.ss_h * g.ss_w;
@@ -849,6 +927,10 @@ static int enqueue_group(vsc_ctx* ctx, Slot* fr, int n, int dtype, const vsc_geo
         fr[i].pcount = 0;
     }
     CU(cudaEventRecord(lead.ev0, lead.stream));
+    if (lead.l_temporal.k > 0) {        // window submission: the filter writes the f32 depth planes the frames read
+        int rc = run_temporal(ctx, lead);
+        if (rc) return rc;
+    }
     ViewSpec vs[TELEA_MAX_VIEWS];
     uchar4* cur[TELEA_MAX_VIEWS];
     for (int i = 0; i < n; i++) {
@@ -909,8 +991,16 @@ static int enqueue_d2h(Slot* fr, int n) {
     return VSC_OK;
 }
 
+// the depth window of a vsc_submit_window call: np consecutive planes, frame i of the submission is plane f0 + i
+struct WindowIn {
+    const void* const* planes;
+    int np, f0, k;
+    double sigma;
+};
+
 static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const* rgb, const void* const* depth, int dtype,
-                             int H, int W, const vsc_params* p, uint8_t* const* out, bool device_io) {
+                             int H, int W, const vsc_params* p, uint8_t* const* out, bool device_io,
+                             const WindowIn* win = nullptr) {
     if (!ctx) return fail(VSC_E_INVALID, "null context");
     const int G = ctx->group_size;
     if (slot < 0 || slot >= (int)ctx->slots.size() / G) return fail(VSC_E_INVALID, "slot %d out of range", slot);
@@ -932,16 +1022,26 @@ static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const
         if ((rc = vsc_encoded_capacity(layout, encode, H, W, &cap))) return rc;
     }
     CU(cudaSetDevice(ctx->device));
+    lead.l_temporal.k = 0;
+    if (win && (rc = ensure_weights(lead, win->k, win->sigma))) return rc;
     const size_t nrgb = (size_t)H * W * 3, ndepth = (size_t)H * W * depth_elem(dtype);
+    float* tplanes[TD_MAX_FRAMES];
     for (int i = 0; i < n; i++) {
         Slot& s = fr[i];
         s.l_rgb = rgb[i]; s.l_depth = depth[i]; s.l_out = out[i]; s.l_host_out = nullptr; s.l_out_bytes = nout;
         s.l_layout = layout; s.l_pixfmt = pixfmt; s.l_matrix = matrix; s.l_encode = encode; s.l_png = nullptr;
+        if (win) {          // the frame reads the filter's f32 plane; its own map reaches the device as a window plane
+            if (s.tdepth.ensure(align_up((size_t)H * W, 4) * 4)) return VSC_E_NOMEM;
+            s.l_depth = tplanes[i] = s.tdepth.as<float>();
+        }
         if (!device_io) {
-            if (s.in_rgb.ensure(nrgb) || s.in_depth.ensure(ndepth) || s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
+            if (s.in_rgb.ensure(nrgb) || (!win && s.in_depth.ensure(ndepth)) || s.out_sbs.ensure(nout)) return VSC_E_NOMEM;
             CU(cudaMemcpyAsync(s.in_rgb.p, rgb[i], nrgb, cudaMemcpyHostToDevice, lead.stream));
-            CU(cudaMemcpyAsync(s.in_depth.p, depth[i], ndepth, cudaMemcpyHostToDevice, lead.stream));
-            s.l_rgb = s.in_rgb.as<uint8_t>(); s.l_depth = s.in_depth.p; s.l_out = s.out_sbs.as<uint8_t>();
+            if (!win) {
+                CU(cudaMemcpyAsync(s.in_depth.p, depth[i], ndepth, cudaMemcpyHostToDevice, lead.stream));
+                s.l_depth = s.in_depth.p;
+            }
+            s.l_rgb = s.in_rgb.as<uint8_t>(); s.l_out = s.out_sbs.as<uint8_t>();
             s.l_host_out = out[i]; s.l_copy_src = s.l_out;
         }
         if (encode == VSC_ENCODE_PNG) {
@@ -961,6 +1061,14 @@ static int submit_group_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const
                 }
             }
         }
+    }
+    if (win) {
+        if ((rc = stage_window(lead, win->planes, win->np, win->f0, n, win->k, dtype, H, W, device_io, tplanes))) {
+            cudaStreamSynchronize(lead.stream);
+            lead.l_temporal.k = 0;
+            return rc;
+        }
+        dtype = VSC_DEPTH_F32;
     }
     rc = enqueue_group(ctx, fr, n, dtype, g, *p);
     if (!rc) rc = enqueue_d2h(fr, n);
@@ -991,6 +1099,32 @@ extern "C" int vsc_submit(vsc_ctx* ctx, int slot, const uint8_t* rgb, const void
 extern "C" int vsc_submit_device(vsc_ctx* ctx, int slot, const uint8_t* d_rgb, const void* d_depth, int dtype, int H, int W,
                                  const vsc_params* p, uint8_t* d_out) {
     return submit_group_impl(ctx, slot, 1, &d_rgb, &d_depth, dtype, H, W, p, &d_out, true);
+}
+
+static int submit_window_impl(vsc_ctx* ctx, int slot, int n, const uint8_t* const* rgb, int n_depth, const void* const* depth,
+                              int first, int dtype, int H, int W, int radius, double sigma, const vsc_params* p,
+                              uint8_t* const* out, bool device_io) {
+    if (!ctx) return fail(VSC_E_INVALID, "null context");
+    if (!depth || n < 1 || n > TD_MAX_FRAMES || n_depth < 1 || first < 0 || first + n > n_depth)
+        return fail(VSC_E_INVALID, "window: frames %d..%d of %d depth planes", first, first + n - 1, n_depth);
+    if (!temporal_args_ok(radius, sigma)) return fail(VSC_E_INVALID, "temporal radius %d / sigma %g out of range ([0,%d], (0,64])", radius, sigma, TD_MAX_RADIUS);
+    if (radius == 0) return submit_group_impl(ctx, slot, n, rgb, depth + first, dtype, H, W, p, out, device_io);
+    if (dtype != VSC_DEPTH_U8 && dtype != VSC_DEPTH_U16) return fail(VSC_E_INVALID, "temporal filtering takes u8 or u16 depth, not dtype %d", dtype);
+    if (H < 1 || W < 1 || (long long)H * W >= (1ll << 31)) return fail(VSC_E_INVALID, "bad frame size %dx%d", W, H);
+    const int lo = std::max(0, first - radius), hi = std::min(n_depth - 1, first + n - 1 + radius);
+    for (int j = lo; j <= hi; j++) if (!depth[j]) return fail(VSC_E_INVALID, "null depth plane %d", j);
+    WindowIn w{depth + lo, hi - lo + 1, first - lo, radius, sigma};
+    return submit_group_impl(ctx, slot, n, rgb, depth + first, dtype, H, W, p, out, device_io, &w);
+}
+extern "C" int vsc_submit_window(vsc_ctx* ctx, int slot, int n, const uint8_t* const* rgb, int n_depth, const void* const* depth,
+                                 int first, int dtype, int H, int W, int radius, double sigma, const vsc_params* p,
+                                 uint8_t* const* out) {
+    return submit_window_impl(ctx, slot, n, rgb, n_depth, depth, first, dtype, H, W, radius, sigma, p, out, false);
+}
+extern "C" int vsc_submit_device_window(vsc_ctx* ctx, int slot, int n, const uint8_t* const* d_rgb, int n_depth,
+                                        const void* const* d_depth, int first, int dtype, int H, int W, int radius, double sigma,
+                                        const vsc_params* p, uint8_t* const* d_out) {
+    return submit_window_impl(ctx, slot, n, d_rgb, n_depth, d_depth, first, dtype, H, W, radius, sigma, p, d_out, true);
 }
 
 static Slot* group_lead(vsc_ctx* ctx, int slot) {
@@ -1508,6 +1642,46 @@ extern "C" int vsc_stage_depth_post(vsc_ctx* ctx, const float* depth, int h, int
     CU(cudaMemcpyAsync(&sc, s.dp_scalars.p, sizeof sc, cudaMemcpyDeviceToHost, s.stream));
     CU(cudaStreamSynchronize(s.stream));
     if (ok) *ok = ord2f(sc.max_ord) - ord2f(sc.min_ord) > 0.f;     // flat map: the reference writes no depth file
+    return VSC_OK;
+}
+
+extern "C" int vsc_stage_temporal_depth(vsc_ctx* ctx, const void* const* depth, int n_depth, int t, int dtype, int H, int W,
+                                        int radius, double sigma, float* out, int* lo, int* hi) {
+    STAGE_BEGIN();
+    if (!depth || !out || n_depth < 1 || t < 0 || t >= n_depth || H < 1 || W < 1 || (long long)H * W >= (1ll << 31))
+        return fail(VSC_E_INVALID, "bad argument");
+    if (dtype != VSC_DEPTH_U8 && dtype != VSC_DEPTH_U16) return fail(VSC_E_INVALID, "temporal filtering takes u8 or u16 depth, not dtype %d", dtype);
+    if (!temporal_args_ok(radius, sigma)) return fail(VSC_E_INVALID, "temporal radius %d / sigma %g out of range ([0,%d], (0,64])", radius, sigma, TD_MAX_RADIUS);
+    const int wlo = std::max(0, t - radius), whi = std::min(n_depth - 1, t + radius);
+    for (int j = wlo; j <= whi; j++) if (!depth[j]) return fail(VSC_E_INVALID, "null depth plane %d", j);
+    const size_t npx = (size_t)H * W;
+    int rc;
+    if ((rc = ensure_weights(s, radius, sigma))) return rc;
+    if (s.tdepth.ensure(align_up(npx, 4) * 4)) return VSC_E_NOMEM;
+    float* o = s.tdepth.as<float>();
+    if ((rc = stage_window(s, depth + wlo, whi - wlo + 1, t - wlo, 1, radius, dtype, H, W, false, &o)) || (rc = run_temporal(ctx, s))) {
+        cudaStreamSynchronize(s.stream);
+        s.l_temporal.k = 0;
+        return rc;
+    }
+    s.l_temporal.k = 0;         // not a window submission of slot 0
+    int w[2];
+    CU(cudaMemcpyAsync(out, o, npx * 4, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaMemcpyAsync(w, s.l_temporal.win, sizeof w, cudaMemcpyDeviceToHost, s.stream));
+    CU(cudaStreamSynchronize(s.stream));
+    if (lo) *lo = wlo + w[0];
+    if (hi) *hi = wlo + w[1];
+    return VSC_OK;
+}
+extern "C" int vsc_debug_i128_to_double(vsc_ctx* ctx, const uint64_t* words, int n, double* out) {
+    if (!ctx || !words || !out || n < 1) return fail(VSC_E_INVALID, "bad argument");
+    CU(cudaSetDevice(ctx->device));
+    Tmp dw, dout;
+    if (dw.alloc((size_t)n * 16) || dout.alloc((size_t)n * 8)) return VSC_E_NOMEM;
+    CU(cudaMemcpy(dw.p, words, (size_t)n * 16, cudaMemcpyHostToDevice));
+    temporal_convert_kernel<<<(n + kThreads - 1) / kThreads, kThreads>>>((const unsigned long long*)dw.p, n, (double*)dout.p);
+    CU(cudaGetLastError());
+    CU(cudaMemcpy(out, dout.p, (size_t)n * 8, cudaMemcpyDeviceToHost));
     return VSC_OK;
 }
 

@@ -20,6 +20,9 @@ side-by-side (default), half side-by-side, top-bottom, half top-bottom or a red-
 (yuv420p, yuv420p10le; BT.709 or BT.601, limited range) instead of rgb24; a YUV format needs `--raw-sink`.
 `--png-encoder gpu` (or the top-level key "sbs_png_encoder") has the GPU encode sbs_*.png and the savers write its bytes
 verbatim; the default `cv2` encodes on the saver threads with cv2.imencode.
+`--temporal-radius K` / `--temporal-sigma S` (or the top-level keys "sbs_temporal_radius" / "sbs_temporal_sigma") filter
+every depth map over its neighbours up to K frames away in the clip before the frame is converted; the default K = 0 is
+the per-frame behaviour.
 """
 from __future__ import annotations
 
@@ -75,6 +78,13 @@ def build_parser() -> ArgumentParser:
     p.add_argument('--png-encoder', choices=PNG_ENCODERS, default=None,
                    help='who encodes sbs_*.png (default: config.json "sbs_png_encoder", else cv2): cv2 on the CPU saver '
                         'threads, or gpu (rgb24 only, not with --raw-sink)')
+    p.add_argument('--temporal-radius', type=int, default=None, metavar='K',
+                   help='filter every depth map over its neighbours up to K frames away, aligned to it and cut at scene '
+                        'changes, against frame-to-frame depth flicker (default: config.json "sbs_temporal_radius", else 0 = '
+                        'off; at most 8)')
+    p.add_argument('--temporal-sigma', type=float, default=None, metavar='S',
+                   help='depth difference, in 8-bit depth units, at which a neighbour\'s weight falls to exp(-1/2) (default: '
+                        'config.json "sbs_temporal_sigma", else 6; in (0, 64])')
     return p
 
 
@@ -123,32 +133,111 @@ def format_refusal(frame_path, layout: str, pixfmt: str):
     return None
 
 
-def _decode_into(item, gen, slot, index, expected):
+def _read_depth(path, size):
+    """A depth map as the loaders use it: grey, resized to size = (height, width) of its frame; None if unreadable."""
+    import cv2
+    from vsc_b200.stereo_core import _resize_depth_to
+    depth = cv2.imread(str(path), cv2.IMREAD_UNCHANGED)
+    if depth is None:
+        return None
+    if depth.ndim == 3:
+        depth = cv2.cvtColor(depth, cv2.COLOR_BGR2GRAY)
+    if depth.shape[:2] != tuple(size):
+        depth = _resize_depth_to(depth, size[1], size[0])
+    return depth
+
+
+def _decode_into(item, gen, slot, index, expected, cache=None):
     """Loader job: decode one (frame, depth) pair.  When the pair has the clip's geometry and depth dtype the colour
     conversion writes straight into the slot's pinned input buffers (no staging copy); otherwise the arrays are
-    returned for the single-frame path.  Returns ('pinned', None) | ('odd', (rgb, depth)) | ('error', message)."""
+    returned for the single-frame path.  Returns ('pinned', None) | ('odd', (rgb, depth)) | ('error', message).
+    With a DepthCache (temporal filter) the depth map comes from the cache and 'pinned' returns it instead of copying it
+    into the slot: the window submission reads it, and its neighbours', from there."""
     import cv2
     import numpy as np
-    from vsc_b200.stereo_core import _resize_depth_to
     try:
         bgr = cv2.imread(str(item[0]), cv2.IMREAD_COLOR)
-        depth = cv2.imread(str(item[1]), cv2.IMREAD_UNCHANGED)
         if bgr is None:
             raise ValueError(f'Could not load RGB: {item[0]}')
+        depth = cache.get(item[1], bgr.shape[:2]) if cache is not None else _read_depth(item[1], bgr.shape[:2])
         if depth is None:
             raise ValueError(f'Could not load depth: {item[1]}')
-        if depth.ndim == 3:
-            depth = cv2.cvtColor(depth, cv2.COLOR_BGR2GRAY)
-        if bgr.shape[:2] != depth.shape[:2]:
-            depth = _resize_depth_to(depth, bgr.shape[1], bgr.shape[0])
         if expected is not None and (bgr.shape[0], bgr.shape[1], depth.dtype.str) == expected:
             prgb, pdepth = gen.pinned_inputs(slot, expected[0], expected[1], np.dtype(expected[2]), index)
             cv2.cvtColor(bgr, cv2.COLOR_BGR2RGB, dst=prgb)
+            if cache is not None:
+                return 'pinned', depth
             np.copyto(pdepth, depth)
             return 'pinned', None
         return 'odd', (cv2.cvtColor(bgr, cv2.COLOR_BGR2RGB), depth)
     except Exception as e:          # reference: the loader logs and skips (sbs_generator.py:229-230)
         return 'error', str(e)
+
+
+class DepthCache:
+    """Depth maps decoded once for the windows of the temporal filter: keyed by (path, frame size), the map as
+    _read_depth gives it (grey, resized to the frame size), or None when it cannot be read.  A map decoded by one
+    loader thread is not decoded again by another that asks for it meanwhile.  Keeps the `capacity` latest maps."""
+
+    def __init__(self, capacity: int):
+        from collections import OrderedDict
+        self._maps = OrderedDict()
+        self._capacity = int(capacity)
+        self._lock = threading.Lock()
+        self.decodes = 0
+
+    def get(self, path, size):
+        from concurrent.futures import Future
+        key = (str(path), tuple(size))
+        with self._lock:
+            f = self._maps.get(key)
+            if f is None:
+                f = self._maps[key] = Future()
+                mine = True
+                while len(self._maps) > self._capacity:
+                    self._maps.popitem(last=False)
+            else:
+                self._maps.move_to_end(key)
+                mine = False
+        if mine:
+            f.set_result(self._decode(path, size))
+        return f.result()
+
+    def _decode(self, path, size):
+        self.decodes += 1
+        try:
+            return _read_depth(path, size)
+        except Exception:       # noqa: BLE001  (an unreadable neighbour ends the window)
+            return None
+
+
+def neighbours(clip, num: int, radius: int, step: int):
+    """Pairs of the frames num + step, num + 2 step, ... within `radius` that the clip has, up to the first gap."""
+    out = []
+    for m in range(1, radius + 1):
+        p = clip.get(num + step * m)
+        if p is None:
+            break
+        out.append(p)
+    return out
+
+
+def window_maps(items, own, clip, radius: int, cache: DepthCache):
+    """(maps, first) of a window submission of the consecutive clip frames `items` with their depth maps `own`: the maps
+    of up to `radius` neighbours on each side, each side ending at the first frame that is missing, fails to decode or
+    does not match the frames' size and dtype."""
+    shape, dt = own[0].shape, own[0].dtype
+
+    def side(step, num):
+        maps = []
+        for p in neighbours(clip, num, radius, step):
+            d = cache.get(p[1], shape)
+            if d is None or d.shape != shape or d.dtype != dt:
+                break
+            maps.append(d)
+        return maps
+    left, right = side(-1, int(items[0][2])), side(1, int(items[-1][2]))
+    return left[::-1] + list(own) + right, len(left)
 
 
 def open_raw_sink(path: str, pairs, layout: str, pixfmt: str = 'rgb24', matrix: str = 'bt709'):
@@ -168,7 +257,8 @@ def open_raw_sink(path: str, pairs, layout: str, pixfmt: str = 'rgb24', matrix: 
 
 def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int, io_threads: int, free_space_mode: str,
                   no_interactive: bool, progress=None, sink=None, sink_index=None, group: int = 4, gen=None,
-                  layout: str = 'sbs', pixfmt: str = 'rgb24', matrix: str = 'bt709', png_encoder: str = 'cv2') -> int:
+                  layout: str = 'sbs', pixfmt: str = 'rgb24', matrix: str = 'bt709', png_encoder: str = 'cv2',
+                  temporal=(0, 6.0), clip=None) -> int:
     """Run `pairs` [(frame_path, depth_path, frame_num)] through one GPU.  Returns frames written.
 
     The pipeline the benchmark times: `slots` frame slots of `group` frames each.  A slot is filled by the loader
@@ -178,11 +268,17 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
     With `sink` (a RawFrameSink shared by all GPUs of the process) frames go to it at position
     `sink_index[frame_num]` instead of into sbs_<n>.png.  `layout`, `pixfmt` and `matrix` set the output of a generator
     made here (a YUV pixfmt only with a sink).  png_encoder='gpu' has that generator encode the PNG files (a caller's
-    generator must then have encode='png'), and the savers write its bytes as they are."""
+    generator must then have encode='png'), and the savers write its bytes as they are.
+    temporal=(radius, sigma) with radius > 0 filters every depth map over its neighbours in `clip` (every pair of the
+    clip, resumed ones included; default `pairs`): submissions then hold consecutive clip frames only, and each depth map
+    is decoded once, through a DepthCache."""
     import cv2
     import numpy as np
     from vsc_b200 import StereoGenerator
-    from vsc_b200.sharder import InOrderPublisher
+    from vsc_b200.sharder import InOrderPublisher, consecutive_chunks
+    radius, sigma = temporal
+    clip_map = {int(p[2]): p for p in (clip if clip is not None else pairs)} if radius else None
+    cache = DepthCache(2 * group * max(2, slots // 2) + 2 * radius + 8) if radius else None
 
     own_gen = gen is None         # a caller may pass a warm generator (n_slots >= slots, group_size >= group) and keep it
     if own_gen:
@@ -259,7 +355,7 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
         for s_ in range(slots):
             for k_ in range(group):
                 gen.pinned_inputs(s_, expected[0], expected[1], np.dtype(expected[2]), k_)
-    chunks = [pairs[i:i + group] for i in range(0, len(pairs), group)]
+    chunks = consecutive_chunks(pairs, group) if radius else [pairs[i:i + group] for i in range(0, len(pairs), group)]
     free_slots = list(range(slots))
     loading = []            # (slot, items, futures), in clip order
     inflight = {}           # slot -> items in the submission
@@ -278,13 +374,42 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
             s = free_slots.pop(0)
             items = chunks[nxt]
             nxt += 1
-            loading.append((s, items, [loaders.submit(_decode_into, it, gen, s, k, expected) for k, it in enumerate(items)]))
+            if radius:          # the frames and their depth maps, and the neighbours' maps the window will read
+                futs = [loaders.submit(_decode_into, it, gen, s, k, expected, cache) for k, it in enumerate(items)]
+                if expected is not None:
+                    halo = neighbours(clip_map, int(items[0][2]), radius, -1) + neighbours(clip_map, int(items[-1][2]), radius, 1)
+                    futs += [loaders.submit(cache.get, p[1], expected[:2]) for p in halo]
+            else:
+                futs = [loaders.submit(_decode_into, it, gen, s, k, expected) for k, it in enumerate(items)]
+            loading.append((s, items, futs))
+
+    def submit_temporal(s, items, results):
+        """Submit a loaded chunk as one window submission, or hand its frames to the single-frame path."""
+        own = [payload for kind, payload in results]
+        if all(kind == 'pinned' for kind, _ in results) and own[0].dtype in (np.uint8, np.uint16):
+            maps, first = window_maps(items, own, clip_map, radius, cache)
+            rgbs = [gen.pinned_inputs(s, expected[0], expected[1], np.dtype(expected[2]), k)[0] for k in range(len(items))]
+            gen.submit_window(s, rgbs, maps, first, params, radius, sigma)
+            inflight[s] = items
+            return
+        for k, (it, (kind, payload)) in enumerate(zip(items, results)):
+            if kind == 'error':
+                skip(it, payload)
+            elif kind == 'pinned':
+                odd.append((it, gen.pinned_inputs(s, expected[0], expected[1], np.dtype(expected[2]), k)[0].copy(), payload))
+            else:
+                odd.append((it, payload[0], payload[1]))
+        free_slots.append(s)
 
     try:
         start_loading()
         while (loading or inflight or odd) and not save_failed.is_set():
             if loading and all(f.done() for f in loading[0][2]):
                 s, items, futs = loading.pop(0)
+                if radius:
+                    submit_temporal(s, items, [f.result() for f in futs[:len(items)]])
+                    start_loading()
+                    continue
                 ok_idx, ok_items = [], []
                 for k, (it, f) in enumerate(zip(items, futs)):
                     kind, payload = f.result()
@@ -303,7 +428,11 @@ def process_shard(pairs, output_dir: Path, params, device_index: int, slots: int
             elif odd and free_slots:
                 it, rgb, depth = odd.pop(0)
                 s = free_slots.pop(0)
-                gen.submit_frames(s, [(rgb, depth)], params)
+                if radius and depth.dtype in (np.uint8, np.uint16):
+                    maps, first = window_maps([it], [depth], clip_map, radius, cache)
+                    gen.submit_window(s, [rgb], maps, first, params, radius, sigma)
+                else:
+                    gen.submit_frames(s, [(rgb, depth)], params)
                 inflight[s] = [it]
             elif inflight:
                 ready = [s for s in inflight if gen.ready(s)]
@@ -338,7 +467,7 @@ def main(argv=None) -> int:
         print(f'ERROR: Workflow directory not found: {args.workflow_path}')
         return 0
     ConfigError, get_path, load_config = _load_config_api()
-    from vsc_b200.workflow import LayoutError, config_layout, config_pixfmt, config_png_encoder
+    from vsc_b200.workflow import LayoutError, config_layout, config_pixfmt, config_png_encoder, config_temporal
     try:
         config = load_config(args.workflow_path)
     except ConfigError as e:
@@ -361,7 +490,15 @@ def main(argv=None) -> int:
         layout = args.layout or config_layout(config)
         cfg_pixfmt, cfg_matrix = config_pixfmt(config)
         png_encoder = args.png_encoder or config_png_encoder(config)
+        cfg_radius, cfg_sigma = config_temporal(config)
     except LayoutError as e:
+        print(f'ERROR: {e}')
+        return 2
+    from vsc_b200.stereo_core import check_temporal
+    try:
+        temporal = check_temporal(cfg_radius if args.temporal_radius is None else args.temporal_radius,
+                                  cfg_sigma if args.temporal_sigma is None else args.temporal_sigma)
+    except ValueError as e:
         print(f'ERROR: {e}')
         return 2
     pixfmt, matrix = args.pixfmt or cfg_pixfmt, args.matrix or cfg_matrix
@@ -413,15 +550,28 @@ def main(argv=None) -> int:
               f'super_sampling={params.super_sampling}, edge_softness={params.edge_softness}, '
               f'smoothing={params.artifact_smoothing}, gamma={params.depth_gamma}, sharpen={params.sharpen}, layout={layout}'
               + (f', pixfmt={pixfmt}, matrix={matrix}' if pixfmt != 'rgb24' else '')
-              + (', png_encoder=gpu' if png_encoder == 'gpu' else ''))
+              + (', png_encoder=gpu' if png_encoder == 'gpu' else '')
+              + (f', temporal_radius={temporal[0]}, temporal_sigma={temporal[1]:g}' if temporal[0] else ''))
 
     finals = [str(output_dir / f'sbs_{p[2]}.png') for p in pairs]
 
-    def free_inputs(i):         # free_space (sbs_generator.py:279-290): only once sbs_<n>.png exists under its final name
+    def free_pair(p):
         if free_space_mode in ('frame', 'all'):
-            Path(pairs[i][0]).unlink(missing_ok=True)
+            Path(p[0]).unlink(missing_ok=True)
         if free_space_mode in ('depth', 'all'):
-            Path(pairs[i][1]).unlink(missing_ok=True)
+            Path(p[1]).unlink(missing_ok=True)
+
+    def free_inputs(i):         # free_space (sbs_generator.py:279-290): only once sbs_<n>.png exists under its final name
+        free_pair(pairs[i])
+    if temporal[0] and free_space_mode != 'none' and not args.raw_sink:
+        # neighbours read a frame's depth map: its inputs go once every frame within the radius has its output
+        from vsc_b200.sharder import DelayedFree
+        by_num = {int(p[2]): p for p in all_pairs}
+        todo = {p[2] for p in pairs}
+        gate = DelayedFree(by_num, [int(p[2]) for p in all_pairs if p[2] not in todo], temporal[0], lambda g: free_pair(by_num[g]))
+
+        def free_inputs(i):     # noqa: F811
+            gate.published(int(pairs[i][2]))
     sink = sink_index = None
     if args.raw_sink:
         if world > 1:
@@ -458,7 +608,7 @@ def main(argv=None) -> int:
             if t:
                 t.start()
             n = process_shard(mine, output_dir, params, local_rank, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                              group=args.group, layout=layout, png_encoder=png_encoder)
+                              group=args.group, layout=layout, png_encoder=png_encoder, temporal=temporal, clip=all_pairs)
             barrier()
             if t:
                 pub.stop()
@@ -473,7 +623,8 @@ def main(argv=None) -> int:
             t.start()
             if g == 1:
                 n = process_shard(pairs, output_dir, params, 0, args.slots, args.io_threads, free_space_mode, args.no_interactive, progress,
-                                  sink, sink_index, args.group, layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder)
+                                  sink, sink_index, args.group, layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder,
+                                  temporal=temporal, clip=all_pairs)
             else:
                 # one worker thread per GPU; each owns a StereoGenerator (its own CUDA context state, streams, pinned ring)
                 results = [0] * g
@@ -483,7 +634,8 @@ def main(argv=None) -> int:
                     try:
                         results[k] = process_shard(shard_items(pairs, g, k), output_dir, params, k, args.slots, args.io_threads,
                                                    free_space_mode, args.no_interactive, progress, sink, sink_index, args.group,
-                                                   layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder)
+                                                   layout=layout, pixfmt=pixfmt, matrix=matrix, png_encoder=png_encoder,
+                                                   temporal=temporal, clip=all_pairs)
                     except BaseException as e:   # noqa: BLE001
                         errors.append(e)
                 ths = [threading.Thread(target=work, args=(k,)) for k in range(g)]

@@ -32,7 +32,9 @@ EXPORTS = [
     'vsc_debug_telea_state', 'vsc_debug_telea_stats', 'vsc_debug_set_telea_capacity', 'vsc_debug_selftest',
     'vsc_layout_shape', 'vsc_set_layout', 'vsc_output_size', 'vsc_set_pixfmt',
     'vsc_set_encode', 'vsc_encoded_capacity', 'vsc_encoded_bytes', 'vsc_stage_png', 'vsc_debug_png_stats',
+    'vsc_submit_window', 'vsc_submit_device_window', 'vsc_stage_temporal_depth', 'vsc_debug_i128_to_double',
 ]
+TEMPORAL_MAX_RADIUS, TEMPORAL_MAX_SIGMA = 8, 64.0
 
 
 class VscParams(C.Structure):
@@ -125,6 +127,11 @@ def load():
     lib.vsc_encoded_bytes.argtypes = [vp, i, i, C.POINTER(C.c_size_t)]
     lib.vsc_stage_png.argtypes = [vp, vp, i, i, vp, C.c_size_t, C.POINTER(C.c_size_t)]
     lib.vsc_debug_png_stats.argtypes = [vp, C.POINTER(C.c_ulonglong)]
+    lib.vsc_submit_window.argtypes = [vp, i, i, C.POINTER(vp), i, C.POINTER(vp), i, i, i, i, i, d, C.POINTER(VscParams), C.POINTER(vp)]
+    lib.vsc_submit_device_window.argtypes = [vp, i, i, C.POINTER(vp), i, C.POINTER(vp), i, i, i, i, i, d, C.POINTER(VscParams),
+                                             C.POINTER(vp)]
+    lib.vsc_stage_temporal_depth.argtypes = [vp, C.POINTER(vp), i, i, i, i, i, i, d, vp, C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    lib.vsc_debug_i128_to_double.argtypes = [vp, vp, i, vp]
     if lib.vsc_abi_version() != 1:
         raise ImportError('libvsc_b200.so ABI version mismatch')
     _lib = lib

@@ -21,8 +21,8 @@ import threading
 import time
 from typing import Callable, List, Optional, Sequence, Tuple
 
-__all__ = ['contiguous_ranges', 'block_cyclic', 'shard_items', 'InOrderPublisher', 'RawFrameSink', 'dist_env', 'barrier',
-           'all_reduce_max']
+__all__ = ['contiguous_ranges', 'block_cyclic', 'shard_items', 'consecutive_chunks', 'DelayedFree', 'InOrderPublisher',
+           'RawFrameSink', 'dist_env', 'barrier', 'all_reduce_max']
 
 
 def contiguous_ranges(n: int, world: int) -> List[Tuple[int, int]]:
@@ -48,6 +48,48 @@ def shard_items(items: Sequence, world: int, rank: int, block: int = 16, mode: s
         a, b = contiguous_ranges(len(items), world)[rank]
         return list(items[a:b])
     return [items[i] for i in block_cyclic(len(items), world, rank, block)]
+
+
+def consecutive_chunks(items: Sequence, group: int, number: Callable = lambda it: int(it[2])) -> list:
+    """`items` cut into chunks of at most `group` consecutive clip frames: a chunk never spans a gap in the frame
+    numbers, so it never straddles a shard block or frames that a resumed run skips."""
+    chunks: list = []
+    run: list = []
+    for it in items:
+        if run and (number(it) != number(run[-1]) + 1 or len(run) == group):
+            chunks.append(run)
+            run = []
+        run.append(it)
+    if run:
+        chunks.append(run)
+    return chunks
+
+
+class DelayedFree:
+    """Free-space deletion with temporal filtering: the maps of frame g are read by every frame within `radius` of it,
+    so its inputs go only once every clip frame in [g - radius, g + radius] has its output (published now, or `done`
+    before this run).  Publication is in order, so in a clip without skipped frames this is: once frame g + radius is
+    published.  A resumed run then still finds every map it needs.  `free(number)` deletes the inputs of one frame."""
+
+    def __init__(self, clip_numbers, done_numbers, radius: int, free: Callable[[int], None]):
+        self._clip = set(int(n) for n in clip_numbers)
+        self._done = set(int(n) for n in done_numbers)
+        self._pending: set = set()
+        self._k = int(radius)
+        self._free = free
+        self._lock = threading.Lock()
+
+    def published(self, number: int) -> None:
+        number = int(number)
+        with self._lock:
+            self._done.add(number)
+            self._pending.add(number)
+            ready = [g for g in range(number - self._k, number + self._k + 1) if g in self._pending and
+                     all(x not in self._clip or x in self._done for x in range(g - self._k, g + self._k + 1))]
+            for g in ready:
+                self._pending.discard(g)
+        for g in ready:
+            self._free(g)
 
 
 class InOrderPublisher:

@@ -13,6 +13,9 @@ Additions that the reference does not have (used by the frame loop in sbs_genera
 return the I420 planes of that frame as one [rows * 3 // 2, cols] array, the shape cv2's COLOR_RGB2YUV_I420 uses.
 PNG output (`StereoGenerator(..., encode='png')`, `ENCODINGS`, `encoded_capacity`): every output path returns the PNG file
 of the rgb24 frame, encoded on the GPU, as a 1-D uint8 array of exactly the file's bytes.
+Temporal depth stabilisation (`StereoGenerator.submit_window`, `process_batch(..., temporal=(radius, sigma))`,
+`temporal_depth`): each frame's depth map is filtered over its neighbours within `radius` frames, aligned to it and cut at
+scene boundaries, before the frame is converted (include/vsc_b200.h has the exact filter).
 """
 from __future__ import annotations
 
@@ -232,6 +235,51 @@ def forward_warp_stereo(image, depth, max_disparity: float):
     return back(left), back(lm), back(right), back(rm)
 
 
+TEMPORAL_SIGMA = 6.0       # default sigma of the temporal filter's depth-difference weight, in 8-bit depth units
+
+
+def check_temporal(radius, sigma) -> Tuple[int, float]:
+    """(radius, sigma) of the temporal filter as (int, float); ValueError unless radius is an integer in 0..8 and sigma a
+    number in (0, 64]."""
+    if isinstance(radius, bool) or not isinstance(radius, (int, np.integer)) or not 0 <= radius <= _lib.TEMPORAL_MAX_RADIUS:
+        raise ValueError(f'temporal radius must be an integer in [0, {_lib.TEMPORAL_MAX_RADIUS}], got {radius!r}')
+    if isinstance(sigma, bool) or not isinstance(sigma, (int, float, np.integer, np.floating)) \
+            or not 0.0 < float(sigma) <= _lib.TEMPORAL_MAX_SIGMA:
+        raise ValueError(f'temporal sigma must be a number in (0, {_lib.TEMPORAL_MAX_SIGMA:g}], got {sigma!r}')
+    return int(radius), float(sigma)
+
+
+def _depth_planes(depths):
+    """Contiguous uint8 / uint16 planes of one size, and their C enum."""
+    planes = [np.ascontiguousarray(d) for d in depths]
+    if not planes:
+        raise ValueError('no depth maps')
+    shape, dt = planes[0].shape, planes[0].dtype
+    if len(shape) != 2 or any(d.shape != shape or d.dtype != dt for d in planes):
+        raise ValueError('the depth maps of a window must be [H, W] arrays of one size and dtype')
+    if dt not in (np.uint8, np.uint16):
+        raise ValueError(f'temporal filtering takes uint8 or uint16 depth maps, not {dt}')
+    return planes, _lib.depth_code(dt)
+
+
+def temporal_depth(depths, t: int, radius: int, sigma: float = TEMPORAL_SIGMA):
+    """The temporal filter alone: depth map t of the consecutive maps `depths`, filtered over its window.  Returns
+    (float32 [H, W] in depth units, lo, hi), where lo..hi (indices into `depths`) is the window that survived the cut
+    rule."""
+    radius, sigma = check_temporal(radius, sigma)
+    planes, code = _depth_planes(depths)
+    if not 0 <= t < len(planes):
+        raise ValueError(f'frame {t} is not one of the {len(planes)} depth maps')
+    h, w = planes[0].shape
+    out = np.empty((h, w), np.float32)
+    lo, hi = C.c_int(), C.c_int()
+    vp = C.c_void_p * len(planes)
+    with _helper_lock:
+        _lib.check(_lib.load().vsc_stage_temporal_depth(_ctx().handle, vp(*[d.ctypes.data for d in planes]), len(planes), int(t),
+                                                        code, h, w, radius, sigma, _lib.ptr(out), C.byref(lo), C.byref(hi)))
+    return out, lo.value, hi.value
+
+
 # ------------------------------------------------------------------------------------------------
 # the generator
 # ------------------------------------------------------------------------------------------------
@@ -366,6 +414,53 @@ class StereoGenerator:
             np.copyto(pdepth, depth_c)
         self.submit_pinned(slot, params, len(frames))
 
+    def submit_window(self, slot: int, frames, depths, first: int, params: StereoParams | None = None,
+                      radius: int = 4, sigma: float = TEMPORAL_SIGMA) -> None:
+        """Enqueue up to `group_size` consecutive clip frames with temporally filtered depth.  `frames` are their rgb
+        arrays, `depths` the consecutive depth maps around them: frame i's own map is depths[first + i], and its window is
+        every map within `radius` of it in `depths` (pass fewer at a clip end or a gap).  The rgb is staged in the slot's
+        pinned buffers; the depth arrays are read in place and must stay untouched until the slot is collected.
+        radius 0 is submit_frames."""
+        radius, sigma = check_temporal(radius, sigma)
+        p = params or self._DEFAULT_PARAMS
+        frames = list(frames)
+        n = len(frames)
+        if not 1 <= n <= self.group_size:
+            raise ValueError(f'a slot takes 1..{self.group_size} frames per submission')
+        if self._pending[slot] is not None:
+            raise RuntimeError(f'slot {slot} has an uncollected frame')
+        planes, code = _depth_planes(depths)
+        if not (0 <= first and first + n <= len(planes)):
+            raise ValueError(f'frames {first}..{first + n - 1} are not all among the {len(planes)} depth maps')
+        h, w = planes[0].shape
+        for i, rgb in enumerate(frames):
+            rgb_c, _, _ = self._check_inputs(rgb, planes[first + i])
+            prgb, _ = self.pinned_inputs(slot, h, w, planes[0].dtype, i)
+            np.copyto(prgb, rgb_c)
+        pins = self._pinned[slot][:n]
+        vp = C.c_void_p * n
+        _lib.check(self._lib.vsc_submit_window(
+            self._ctx.handle, slot, n, vp(*[x[1].array.ctypes.data for x in pins]), len(planes),
+            (C.c_void_p * len(planes))(*[d.ctypes.data for d in planes]), int(first), code, h, w, radius, sigma,
+            C.byref(_lib.make_params(p)), vp(*[x[3].array.ctypes.data for x in pins])))
+        self._pending[slot] = n
+        self._held = getattr(self, '_held', {})
+        self._held[slot] = planes            # keep the maps alive until collect()
+
+    def submit_device_window(self, slot: int, triples, d_depths, first: int, depth_dtype, h: int, w: int,
+                             params: StereoParams | None = None, radius: int = 4, sigma: float = TEMPORAL_SIGMA) -> None:
+        """Device-resident submit_window: `triples` = [(d_rgb, d_out)] raw device pointers (<= group_size), `d_depths` the
+        window's depth maps (raw device pointers), frame i's own map d_depths[first + i]."""
+        radius, sigma = check_temporal(radius, sigma)
+        p = params or self._DEFAULT_PARAMS
+        triples, d_depths = list(triples), list(d_depths)
+        n = len(triples)
+        vp = C.c_void_p * n
+        _lib.check(self._lib.vsc_submit_device_window(
+            self._ctx.handle, slot, n, vp(*[t[0] for t in triples]), len(d_depths), (C.c_void_p * len(d_depths))(*d_depths),
+            int(first), _lib.depth_code(depth_dtype), h, w, radius, sigma, C.byref(_lib.make_params(p)),
+            vp(*[t[1] for t in triples])))
+
     def collect(self, slot: int, copy: bool = True):
         """Wait for the slot's submission.  Returns the output frame (a list of frames if more than one was
         submitted).  copy=True returns fresh arrays the caller owns (the reference hands its result to another
@@ -474,10 +569,13 @@ class StereoGenerator:
         return [(names[i].decode(), float(ms[i])) for i in range(n)]
 
     def process_batch(self, frames: Iterable[Tuple[np.ndarray, np.ndarray]],
-                      params: StereoParams | None = None) -> List[np.ndarray]:
+                      params: StereoParams | None = None, temporal: Optional[Tuple[int, float]] = None) -> List[np.ndarray]:
         """Run an iterable of (rgb, depth) through all slots, keeping `n_slots * group_size` frames in flight.
-        Results are returned in input order."""
+        Results are returned in input order.  With temporal=(radius, sigma) the frames are consecutive frames of one clip
+        (one size, uint8 or uint16 depth) and every depth map is filtered over its neighbours (submit_window)."""
         frames = list(frames)
+        if temporal is not None:
+            return self._process_batch_temporal(frames, params, *check_temporal(*temporal))
         out: List[Optional[np.ndarray]] = [None] * len(frames)
         g = self.group_size
         chunks = [list(range(i, min(i + g, len(frames)))) for i in range(0, len(frames), g)]
@@ -506,6 +604,31 @@ class StereoGenerator:
                 inflight.append((slot, part))
         for slot, ids in inflight:
             harvest(slot, ids)
+        return out  # type: ignore[return-value]
+
+    def _process_batch_temporal(self, frames, params, radius: int, sigma: float) -> List[np.ndarray]:
+        depths, _ = _depth_planes([f[1] for f in frames]) if frames else ([], None)
+        out: List[Optional[np.ndarray]] = [None] * len(frames)
+        inflight: List[Tuple[int, range]] = []
+        free = list(range(self.n_slots))
+        for a in range(0, len(frames), self.group_size):
+            idxs = range(a, min(a + self.group_size, len(frames)))
+            if not free:
+                slot = self.wait_any([s for s, _ in inflight])
+                ids = next(x for s, x in inflight if s == slot)
+                inflight.remove((slot, ids))
+                res = self.collect(slot)
+                for i, r in zip(ids, res if isinstance(res, list) else [res]):
+                    out[i] = r
+                free.append(slot)
+            slot = free.pop(0)
+            lo, hi = max(0, idxs[0] - radius), min(len(frames) - 1, idxs[-1] + radius)
+            self.submit_window(slot, [frames[i][0] for i in idxs], depths[lo:hi + 1], idxs[0] - lo, params, radius, sigma)
+            inflight.append((slot, idxs))
+        for slot, ids in inflight:
+            res = self.collect(slot)
+            for i, r in zip(ids, res if isinstance(res, list) else [res]):
+                out[i] = r
         return out  # type: ignore[return-value]
 
     def last_frame_ms(self, slot: int = 0) -> float:

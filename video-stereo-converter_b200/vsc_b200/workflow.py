@@ -10,7 +10,8 @@ stereo_core.LAYOUTS, default "sbs").  It sits at the top level because the refer
 top-level keys while the reference builds StereoParams from the whole `stereo` block.  So do the optional
 "sbs_pixfmt" (pixel format of the frames, one of stereo_core.PIXFMTS, default "rgb24") and "sbs_matrix" (YUV matrix, one
 of stereo_core.MATRICES, default "bt709"), and "sbs_png_encoder" (who encodes sbs_*.png, one of PNG_ENCODERS, default
-"cv2").
+"cv2"), and "sbs_temporal_radius" / "sbs_temporal_sigma" (temporal depth filter, radius 0..8 frames, default 0 = off;
+sigma in (0, 64], default 6).
 """
 from __future__ import annotations
 
@@ -25,6 +26,7 @@ PIXFMT_KEY, MATRIX_KEY = 'sbs_pixfmt', 'sbs_matrix'
 PNG_ENCODER_KEY = 'sbs_png_encoder'
 # who encodes sbs_*.png: 'cv2' (cv2.imencode on the saver threads) or 'gpu' (the library's PNG encoding, written verbatim)
 PNG_ENCODERS = ('cv2', 'gpu')
+TEMPORAL_RADIUS_KEY, TEMPORAL_SIGMA_KEY = 'sbs_temporal_radius', 'sbs_temporal_sigma'
 
 
 class ConfigError(Exception):
@@ -65,6 +67,17 @@ def config_png_encoder(cfg: Dict) -> str:
     return v
 
 
+def config_temporal(cfg: Dict):
+    """(radius, sigma) of the temporal depth filter a config asks for: top-level "sbs_temporal_radius" (an integer in
+    0..8, default 0 = off) and "sbs_temporal_sigma" (a number in (0, 64], default 6)."""
+    from .stereo_core import TEMPORAL_SIGMA, check_temporal
+    r, s = cfg.get(TEMPORAL_RADIUS_KEY, 0), cfg.get(TEMPORAL_SIGMA_KEY, TEMPORAL_SIGMA)
+    try:
+        return check_temporal(r, s)
+    except ValueError as e:
+        raise LayoutError(f"Invalid '{TEMPORAL_RADIUS_KEY}' {r!r} / '{TEMPORAL_SIGMA_KEY}' {s!r}: {e}")
+
+
 def load_config(workflow_path) -> Dict:
     f = Path(workflow_path) / 'config.json'
     if not f.exists():
@@ -88,6 +101,7 @@ def load_config(workflow_path) -> Dict:
     config_layout(cfg)
     config_pixfmt(cfg)
     config_png_encoder(cfg)
+    config_temporal(cfg)
     return cfg
 
 
