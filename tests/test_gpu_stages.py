@@ -21,7 +21,14 @@ def _params(**kw):
     return p, _lib.make_params(p)
 
 
-@pytest.mark.parametrize('h,w,dw', [(37, 160, 270), (24, 1920, 2030), (9, 3840, 3949), (11, 100, 137), (8, 64, 64)])
+# Rows of 100..115 pixels: every row-length residue mod 16 bytes, at H = 1 (the last row of a buffer is read with LSU
+# loads) and at H = 17 (rows 0..15 are staged by TMA from g & ~15; an odd width puts their starts on every residue).
+# Widths 100 and 112 at H >= 2 have the residues of the cases above.
+LANCZOS_CASES = [(37, 160, 270), (24, 1920, 2030), (9, 3840, 3949), (11, 100, 137), (8, 64, 64)]
+LANCZOS_EDGE_CASES = [(h, w, w + 37) for h in (1, 17) for w in range(100, 116) if h == 1 or w not in (100, 112)]
+
+
+@pytest.mark.parametrize('h,w,dw', LANCZOS_CASES + LANCZOS_EDGE_CASES)
 def test_lanczos_all_dtypes(ctx, h, w, dw):
     rng = np.random.default_rng(h * w)
     lib = _lib.load()
@@ -51,7 +58,7 @@ def _oracle_depth(depth_st, hs, ws, p):
     return d
 
 
-@pytest.mark.parametrize('h,sw,kw', [
+DEPTH_CASES = [
     (120, 270, {}),
     (90, 200, dict(super_sampling=2.5, edge_softness=3.0, depth_gamma=0.5)),
     (100, 180, dict(super_sampling=1.0, edge_softness=0.0, depth_gamma=1.0)),
@@ -60,10 +67,48 @@ def _oracle_depth(depth_st, hs, ws, p):
     (200, 333, dict(super_sampling=1.7, edge_softness=30.0, depth_gamma=1.3)),
     (81, 111, {}),                                                                   # odd super-sampled width (333): scalar stores, last column unpaired
     (75, 131, dict(super_sampling=1.0, edge_softness=10.0, depth_gamma=0.7)),        # odd width, generic tap count
-])
+]
+# Every generic tap count k = 5..29 with and without the upsample, depth_point_kernel at gamma 2 and 3, and 1x grids
+# at the 64-pixel tile edges (64k - 1, 64k, 64k + 1) and below one tile.  Their depth maps have flat areas at the
+# minimum and the maximum, so gamma meets the clamp at 0.001 and x = 1.
+DEPTH_EDGE_CASES = [
+    (63, 127, dict(super_sampling=1.0, edge_softness=5 / 6, depth_gamma=2.0)),
+    (64, 128, dict(super_sampling=1.0, edge_softness=7 / 6, depth_gamma=3.0)),
+    (65, 129, dict(super_sampling=1.0, edge_softness=9 / 6, depth_gamma=1.0)),
+    (127, 63, dict(super_sampling=1.0, edge_softness=11 / 6, depth_gamma=0.5)),
+    (128, 65, dict(super_sampling=1.0, edge_softness=13 / 6, depth_gamma=0.37)),
+    (129, 64, dict(super_sampling=1.0, edge_softness=15 / 6, depth_gamma=3.0)),
+    (20, 50, dict(super_sampling=1.0, edge_softness=17 / 6, depth_gamma=2.0)),
+    (40, 191, dict(super_sampling=1.0, edge_softness=19 / 6, depth_gamma=0.2)),
+    (45, 70, dict(super_sampling=1.0, edge_softness=21 / 6, depth_gamma=1.0)),
+    (50, 100, dict(super_sampling=1.0, edge_softness=23 / 6, depth_gamma=0.8)),
+    (33, 65, dict(super_sampling=1.0, edge_softness=25 / 6, depth_gamma=1.6)),
+    (60, 130, dict(super_sampling=1.0, edge_softness=27 / 6, depth_gamma=2.0)),
+    (31, 129, dict(super_sampling=1.0, edge_softness=29 / 6, depth_gamma=3.0)),
+    (30, 60, dict(super_sampling=2.0, edge_softness=5 / 6, depth_gamma=3.0)),
+    (25, 51, dict(super_sampling=2.5, edge_softness=7 / 6, depth_gamma=2.0)),
+    (32, 64, dict(super_sampling=1.5, edge_softness=9 / 6, depth_gamma=1.0)),
+    (21, 43, dict(super_sampling=3.0, edge_softness=11 / 6, depth_gamma=0.6)),
+    (40, 80, dict(super_sampling=1.6, edge_softness=13 / 6, depth_gamma=3.0)),
+    (22, 40, dict(super_sampling=2.9, edge_softness=15 / 6, depth_gamma=0.25)),
+    (35, 71, dict(super_sampling=2.0, edge_softness=17 / 6, depth_gamma=2.0)),
+    (18, 45, dict(super_sampling=4.0, edge_softness=21 / 6, depth_gamma=1.0)),
+    (27, 60, dict(super_sampling=2.2, edge_softness=23 / 6, depth_gamma=0.4)),
+    (29, 66, dict(super_sampling=1.9, edge_softness=25 / 6, depth_gamma=3.0)),
+    (31, 70, dict(super_sampling=2.0, edge_softness=27 / 6, depth_gamma=1.3)),
+    (33, 65, dict(super_sampling=2.0, edge_softness=29 / 6, depth_gamma=2.0)),
+    (50, 90, dict(super_sampling=1.0, edge_softness=0.0, depth_gamma=2.0)),
+    (26, 70, dict(super_sampling=2.0, edge_softness=0.0, depth_gamma=3.0)),
+]
+
+
+@pytest.mark.parametrize('h,sw,kw', DEPTH_CASES + DEPTH_EDGE_CASES)
 def test_depth_front(ctx, h, sw, kw):
     p, cp = _params(**kw)
     depth_st = make_depth(h, sw, seed=h, dtype=np.uint16).astype(np.float32)
+    if (h, sw, kw) in DEPTH_EDGE_CASES:
+        depth_st[:h // 4] = 0
+        depth_st[-h // 4:, :sw // 3] = 65535
     ss = p.super_sampling > 1.0
     hs, ws = (int(h * p.super_sampling), int(sw * p.super_sampling)) if ss else (h, sw)
     out = np.empty((hs, ws), np.float32)
@@ -95,10 +140,20 @@ def _oracle_warp_u8(rgb_st, depth_ss, hs, ws, md, ss, scale255=False):
     return res
 
 
-@pytest.mark.parametrize('h,sw,s,md,kind', [
+WARP_CASES = [
     (60, 200, 3.0, 50.0, 'random'), (45, 333, 1.0, 17.5, 'ties'), (30, 500, 2.0, 100.0, 'ramp'),
     (40, 1500, 1.0, 100.0, 'random'), (33, 410, 2.5, 5.0, 'discs'), (20, 2300, 1.0, 63.5, 'discs'),
-])
+]
+# ss_w on the 1024-target segment edges (1024, 1025, 2048, 2049, 3073), md = 0, and a halo ceil(md) + 1 = 101 wider
+# than the 96-target segment of a 90-pixel row
+WARP_EDGE_CASES = [
+    (4, 1024, 1.0, 30.0, 'random'), (3, 1025, 1.0, 0.0, 'random'), (3, 2048, 1.0, 12.25, 'ties'),
+    (2, 2049, 1.0, 100.0, 'ramp'), (2, 3073, 1.0, 40.0, 'discs'), (12, 90, 1.0, 100.0, 'random'),
+]
+WARP_SCALE255_CASE = (24, 120, 3.0, 20.0)
+
+
+@pytest.mark.parametrize('h,sw,s,md,kind', WARP_CASES + WARP_EDGE_CASES)
 def test_warp_bit_exact(ctx, h, sw, s, md, kind):
     rng = np.random.default_rng(int(md * 10) + h)
     ss = s > 1.0
@@ -126,7 +181,7 @@ def test_warp_bit_exact(ctx, h, sw, s, md, kind):
 
 def test_warp_scale255_branch(ctx):
     """stereo_core.py:404-407: a view whose float max is <= 1.0 is multiplied by 255 before the uint8 cast."""
-    h, sw, s, md = 24, 120, 3.0, 20.0
+    h, sw, s, md = WARP_SCALE255_CASE
     hs, ws = int(h * s), int(sw * s)
     rng = np.random.default_rng(5)
     rgb_st = rng.integers(0, 2, (h, sw, 3), dtype=np.uint8)
@@ -297,10 +352,32 @@ def test_inpaint_real_warp_masks(ctx):
         assert np.array_equal(out, ref), f'{side}: {(out != ref).any(axis=2).sum()} px differ'
 
 
-@pytest.mark.parametrize('hs,ws,h,w,lc,rc,cw,sharp', [
+BACKEND_CASES = [
     (360, 810, 120, 160, 135, 195, 480, 14.0), (225, 540, 90, 150, 40, 70, 375, 6.5), (100, 245, 100, 180, 37, 27, 180, 14.0),
     (360, 810, 120, 160, 135, 195, 480, 0.0), (130, 300, 100, 211, 3, 9, 274, 16.0), (256, 700, 64, 150, 50, 38, 600, 1.0),
-])
+]
+
+
+def _backend_edge_cases():
+    """K = 0 (2.5x), 1x, 2, 3 and 4, each on outputs of all-FULL tiles, partial tiles along x (W % 32 != 0), along y
+    (H % 8 != 0) and both, with and without sharpening; the sharpened crops touch both edges of the views.  The
+    combinations BACKEND_CASES already has are left out."""
+    have = {(2.5, 20, 70, True), (1, 20, 70, True), (3, 16, 64, True), (3, 16, 64, False), (4, 16, 70, True)}
+    cases = []
+    for s in (2.5, 1, 2, 3, 4):
+        for h, w in ((16, 64), (16, 70), (20, 64), (20, 70)):
+            hs, cw = int(h * s), int(w * s)
+            if (s, h, w, True) not in have:
+                cases.append((hs, cw + 40, h, w, 0, 40, cw, 3.5 + s))
+            if (s, h, w, False) not in have:
+                cases.append((hs, cw + 40, h, w, 17, 23, cw, 0.0))
+    return cases
+
+
+BACKEND_EDGE_CASES = _backend_edge_cases()
+
+
+@pytest.mark.parametrize('hs,ws,h,w,lc,rc,cw,sharp', BACKEND_CASES + BACKEND_EDGE_CASES)
 def test_backend_bit_exact(ctx, hs, ws, h, w, lc, rc, cw, sharp):
     rng = np.random.default_rng(hs + w)
     left = make_rgb(hs, ws, seed=1)
